@@ -10,8 +10,9 @@ in the device-resident arm and in the end-to-end arm alike.
     python bench.py [--gpus N] [--steps K] [--warmup W]        # this repo's CUDA path
     python bench.py --impl reference ...                        # the CPU path on the host cores (same config object)
     one GPU: BASELINE configs[1] (1k grid, N = 30); under torchrun: configs[2], the FIXED 16k x N = 50 sweep strong-scaled
+    --dump-outputs DIR: also write the results of the last timed step as DIR/<name>.npy (see dump_outputs)
 
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0).  Writes nothing into the checkout, which may be read-only.
 """
 import argparse
 import json
@@ -23,6 +24,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # (no __pycache__ in the checkout for the modules imported below)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -255,6 +257,35 @@ def run_reference(args):
     print(json.dumps(line))
 
 
+def sweep_records(gathered, total, world):
+    """All-gathered result records [world, Bmax, nx + 3] (rank-major; each rank's interleaved shard padded to Bmax)
+    -> x, f, status, iters of the whole sweep in sweep order."""
+    import landing_controller_b200 as lc
+    parts = [gathered[r, :len(lc.shard_indices(total, world, r))] for r in range(world)]
+    ordered = np.empty((total, gathered.shape[2]))
+    ordered[lc.unshard_order(total, world)] = np.concatenate(parts)
+    return lc.unpack_records(ordered)
+
+
+DUMP_LIMIT = 64 << 20  # bytes written by --dump-outputs
+
+
+def dump_outputs(path, x, f, status, iters):
+    """What the timed path returned to its caller in the last step, as float64 arrays <path>/<name>.npy: x [B, nx]
+    (x*), f (f*), status, iters, and scenario (the index in the sweep of each row).  The sweep is fixed by the
+    arguments, so two builds run with the same arguments can be compared output for output.  When the whole sweep is
+    larger than DUMP_LIMIT a fixed, seeded sample of its scenarios is written."""
+    B, nx = x.shape
+    keep = np.arange(B)
+    row_bytes = 8 * (nx + 4)
+    if B * row_bytes > DUMP_LIMIT:
+        keep = np.sort(np.random.default_rng(0).choice(B, DUMP_LIMIT // row_bytes, replace=False))
+    os.makedirs(path, exist_ok=True)
+    out = {"x": x[keep], "f": f[keep], "status": status[keep], "iters": iters[keep], "scenario": keep}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def iter_stats(its, st):
     its = np.asarray(its, dtype=np.float64)
     q = lambda f: float(np.percentile(its, f))
@@ -278,7 +309,13 @@ def main():
                     help="NOT the default: landing_options.restart_mu for both arms (DESIGN.md 3); 0 = mu_init")
     ap.add_argument("--no-one-gpu-base", action="store_true",
                     help="N > 1: skip the 1-GPU solve of the same fixed workload on rank 0 (strong-scaling base)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step (x*, f*, status, iters per scenario) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path, not of --impl reference")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -403,6 +440,12 @@ def main():
         all_st = np.concatenate([g[r, :len(lc.shard_indices(cfg["total"], world, r)), nx + 1] for r in range(world)])
     else:
         all_its, all_st = its, st
+    last = None
+    if args.dump_outputs and rank == 0:  # (the end-to-end arm below overwrites the device buffers when N > 1)
+        if world > 1:
+            last = sweep_records(g, cfg["total"], world)
+        else:
+            last = dict(x=x_d.cpu().numpy(), f=f_d.cpu().numpy(), status=st, iters=its)
 
     for _ in range(min(args.warmup, 1)):
         step_e2e()
@@ -517,6 +560,8 @@ def main():
                 "kkt_iters_per_s": float(r["iters"].sum()) / dt,
                 "sample": "%d of %d scenarios (every %d-th), %.1f s; IPOPT substitute oracle/ip_ref.c (%s), OpenMP over scenarios"
                           % (len(sub), B, stride, dt, cpu_flags())}
+        if last is not None:
+            dump_outputs(args.dump_outputs, last["x"], last["f"], last["status"], last["iters"])
         print(json.dumps(line))
     if world > 1:
         dist.barrier()

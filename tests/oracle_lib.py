@@ -4,9 +4,12 @@ the compiled reference C (oracle/_ref/landingCtrller_IPOPT.so).
 TEST INFRASTRUCTURE: imported only by tests/, bench.py's cpu_baseline/reference legs and
 __graft_entry__.smoke().  The product package never imports this module.
 """
+import atexit
 import ctypes
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -31,19 +34,21 @@ def build_oracle(force=False):
     return ORACLE_SO
 
 
-FAST_SO = os.path.join(ORACLE_DIR, "liboracle_fast.so")
-
-
 def build_oracle_fast():
     """The -O3 -march=native build used by the TIMED CPU arm of bench.py (never by the parity tests): always rebuilt on
-    the host that runs the bench, because -march=native code from another machine may not run here.  Falls back to the
-    bit-reproducible build (and says so) when there is no compiler."""
+    the host that runs the bench, because -march=native code from another machine may not run here.  It goes to a
+    temporary directory (removed at exit), so that the bench writes nothing into the checkout, which may be read-only.
+    When that build fails, falls back to the bit-reproducible build and says so, with the error, in the returned label."""
     try:
-        subprocess.check_call(["make", "-B", "-C", ORACLE_DIR, "liboracle_fast.so"], stdout=subprocess.DEVNULL,
-                              stderr=subprocess.DEVNULL)
-        return FAST_SO, "gcc -O3 -march=native -fopenmp (built on this host)"
-    except Exception:
-        return build_oracle(), "gcc -O2 -ffp-contract=off -fopenmp (no compiler on this host for the -O3 build)"
+        tmp = tempfile.mkdtemp(prefix="landing_oracle_")
+        atexit.register(shutil.rmtree, tmp, True)
+        fast_so = os.path.join(tmp, "liboracle_fast.so")
+        subprocess.run(["make", "-C", ORACLE_DIR, "fast", "FAST_SO=" + fast_so], check=True, capture_output=True,
+                       text=True)
+        return fast_so, "gcc -O3 -march=native -fopenmp (built on this host)"
+    except (OSError, subprocess.CalledProcessError) as e:
+        why = (getattr(e, "stderr", None) or "").strip().splitlines() or [str(e)]
+        return build_oracle(), "gcc -O2 -ffp-contract=off -fopenmp (the -O3 build failed: %s)" % why[-1]
 
 
 class Plan(ctypes.Structure):

@@ -72,7 +72,8 @@ def test_kat0_from_survey(o21, golden):
     assert abs(H.sum() - 560.1979584000001) < 1e-9 and abs(np.abs(H).sum() - 2607.579796) < 1e-9
 
 
-@pytest.mark.skipif(not have_ref(), reason="compiled reference C not present (GPU box)")
+@pytest.mark.skipif(not have_ref(), reason="compiled reference C not present (oracle/_ref, built by `make -C oracle ref` "
+                                           "from the reference's own landingCtrller_IPOPT.c)")
 def test_live_reference_random(o21):
     ref = CasadiLib(REF_SO)
     rng = np.random.default_rng(7)

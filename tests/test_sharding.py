@@ -99,3 +99,58 @@ def test_reference_arm_line_schema():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["value"] == line["value"] > 0
     for k in ("metric", "n_gpus", "steps", "warmup", "ms_per_step", "scaling", "dtype", "data", "config"):
         assert k in line
+
+
+def test_bench_dump_outputs_whole_and_sampled(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 .npy files, the whole sweep when it fits the size limit, otherwise the same
+    seeded sample of scenarios on every call."""
+    import sys
+    monkeypatch.setattr(sys, "dont_write_bytecode", sys.dont_write_bytecode)  # (bench sets it on import)
+    import bench
+    B, nx = 50, 10
+    x = np.arange(B * nx, dtype=np.float64).reshape(B, nx)
+    f, st, it = np.arange(B) * 0.5, np.arange(B, dtype=np.int32) % 5, np.arange(B, dtype=np.int32)
+    load = lambda d: {n: np.load(os.path.join(d, n + ".npy")) for n in ("x", "f", "status", "iters", "scenario")}
+    bench.dump_outputs(str(tmp_path / "all"), x, f, st, it)
+    a = load(str(tmp_path / "all"))
+    assert all(v.dtype == np.float64 for v in a.values())
+    assert np.array_equal(a["x"], x) and np.array_equal(a["status"], st) and np.array_equal(a["scenario"], np.arange(B))
+    monkeypatch.setattr(bench, "DUMP_LIMIT", 8 * (nx + 4) * 12)  # room for 12 scenarios
+    bench.dump_outputs(str(tmp_path / "s1"), x, f, st, it)
+    bench.dump_outputs(str(tmp_path / "s2"), x, f, st, it)
+    s1, s2 = load(str(tmp_path / "s1")), load(str(tmp_path / "s2"))
+    ids = s1["scenario"].astype(int)
+    assert len(ids) == 12 and len(np.unique(ids)) == 12 and all(np.array_equal(s1[n], s2[n]) for n in s1)
+    assert sum(v.nbytes for v in s1.values()) <= bench.DUMP_LIMIT
+    assert np.array_equal(s1["x"], x[ids]) and np.array_equal(s1["f"], f[ids]) and np.array_equal(s1["iters"], it[ids])
+
+
+def test_bench_sweep_records_undo_the_interleaved_all_gather(monkeypatch):
+    """bench.py --dump-outputs under torchrun: the padded, rank-major all-gathered records back in sweep order."""
+    import sys
+    monkeypatch.setattr(sys, "dont_write_bytecode", sys.dont_write_bytecode)
+    import bench
+    n, nx = 37, 4
+    for world in (1, 2, 3, 8):
+        x = np.arange(n * nx, dtype=np.float64).reshape(n, nx) + 0.25
+        rec = lc.pack_records(x, np.arange(n) * 1.5, np.arange(n) % 5, np.arange(n) + 7)
+        bmax = -(-n // world)
+        gathered = np.full((world, bmax, nx + 3), np.nan)  # padding rows must never be read
+        for r in range(world):
+            ids = lc.shard_indices(n, world, r)
+            gathered[r, :len(ids)] = rec[ids]
+        out = bench.sweep_records(gathered, n, world)
+        ref = lc.unpack_records(rec)
+        assert all(np.array_equal(out[k], ref[k]) for k in ("x", "f", "status", "iters"))
+
+
+def test_fast_oracle_fallback_names_the_failure(monkeypatch):
+    """The timed CPU arm's -O3 build falls back to the -O2 library only with the reason in its label."""
+    import tempfile
+    import oracle_lib
+
+    def no_tmp(**kw):
+        raise PermissionError("temporary directory not writable")
+    monkeypatch.setattr(tempfile, "mkdtemp", no_tmp)
+    path, how = oracle_lib.build_oracle_fast()
+    assert path == oracle_lib.ORACLE_SO and "-O2" in how and "temporary directory not writable" in how
