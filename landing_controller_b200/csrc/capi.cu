@@ -46,84 +46,143 @@ struct landing_ctx {
   cudaStream_t stream = nullptr;
   int* d_maps = nullptr;
   long long launches = 0;
-  // grow-only device staging for host-buffer calls
-  void* stage = nullptr;
-  size_t stage_bytes = 0;
-  void* pin = nullptr;  // mapped pinned host buffer of small LANDING_HOST evaluation calls (zero-copy)
-  size_t pin_bytes = 0;
-  // grow-only scratch for the transposed (SoA) copies of AoS batches
-  void* tr = nullptr;
-  size_t tr_bytes = 0;
+  DeviceBuf stage;  // device staging of host-buffer calls (stage_in)
+  MappedBuf pin;    // the same for small evaluation calls, zero-copy
+  DeviceBuf tr;     // transposed (SoA) copies of AoS batches (aos_to_soa)
   SolverWorkspace ws;
   // knot spacings of the current call: pinned host staging + device copy (landing_problem.dt or uniform)
-  double* h_dt = nullptr;
-  double* d_dt = nullptr;
+  PinnedBuf h_dt;
+  DeviceBuf d_dt;
   // contact schedule of the current call (formulation 1): bit mask per knot
-  unsigned char* h_cs = nullptr;
-  unsigned char* d_cs = nullptr;
+  PinnedBuf h_cs;
+  DeviceBuf d_cs;
   // kino-dynamic NLP (landing_kino_eval_batch): host plan and its device tables, made on first use
   std::shared_ptr<const KinoPlan> kino;
   int* d_kino = nullptr;
 };
 
 // dt[0..N-2] of this call on the device (stream-ordered): the caller's vector or the uniform T/(N-1)
-static int stage_dt(landing_ctx* c, const landing_problem* pb) {
+static int stage_dt(landing_ctx* c, const double* dt, double T) {
   const int K = c->N - 1;
-  if (!c->h_dt) CU(cudaMallocHost(&c->h_dt, sizeof(double) * K));
-  if (!c->d_dt) CU(cudaMalloc(&c->d_dt, sizeof(double) * K));
-  CU(cudaStreamSynchronize(c->stream));  // the previous call's copy out of h_dt has completed
+  CU(c->h_dt.reserve(sizeof(double) * K));
+  CU(c->d_dt.reserve(sizeof(double) * K));
+  CU(cudaStreamSynchronize(c->stream));  // the previous call's copies out of h_dt and h_cs (stage_cs) have completed
   for (int k = 0; k < K; k++) {
-    const double h = pb->dt ? pb->dt[k] : pb->T / (double)K;
+    const double h = dt ? dt[k] : T / (double)K;
     if (!(h > 0.0)) return fail(LANDING_ERR_ARG, "landing_problem: knot spacings must be positive");
-    c->h_dt[k] = h;
+    c->h_dt.as<double>()[k] = h;
   }
-  CU(cudaMemcpyAsync(c->d_dt, c->h_dt, sizeof(double) * K, cudaMemcpyHostToDevice, c->stream));
-  if (pb->formulation == 1) {
-    if (!pb->cs) return fail(LANDING_ERR_ARG, "landing_problem: formulation 1 needs the contact schedule cs[4 (N-1)]");
-    if (!(pb->delta_c > 0.0)) return fail(LANDING_ERR_ARG, "landing_problem: delta_c must be positive");
-    if (!c->h_cs) CU(cudaMallocHost(&c->h_cs, K));
-    if (!c->d_cs) CU(cudaMalloc(&c->d_cs, K));
-    for (int k = 0; k < K; k++) {
-      unsigned m = 0;
-      for (int l = 0; l < 4; l++) m |= (pb->cs[4 * k + l] != 0) << l;
-      c->h_cs[k] = (unsigned char)m;
+  CU(cudaMemcpyAsync(c->d_dt.as<double>(), c->h_dt.as<double>(), sizeof(double) * K, cudaMemcpyHostToDevice, c->stream));
+  return LANDING_OK;
+}
+
+// the contact schedule of formulation 1 on the device (after stage_dt, whose synchronisation covers h_cs)
+static int stage_cs(landing_ctx* c, const landing_problem* pb) {
+  if (pb->formulation == 0) return LANDING_OK;
+  if (pb->formulation != 1) return fail(LANDING_ERR_ARG, "landing_problem: formulation must be 0 or 1");
+  if (!pb->cs) return fail(LANDING_ERR_ARG, "landing_problem: formulation 1 needs the contact schedule cs[4 (N-1)]");
+  if (!(pb->delta_c > 0.0)) return fail(LANDING_ERR_ARG, "landing_problem: delta_c must be positive");
+  const int K = c->N - 1;
+  CU(c->h_cs.reserve(K));
+  CU(c->d_cs.reserve(K));
+  for (int k = 0; k < K; k++) {
+    unsigned m = 0;
+    for (int l = 0; l < 4; l++) m |= (pb->cs[4 * k + l] != 0) << l;
+    c->h_cs.as<unsigned char>()[k] = (unsigned char)m;
+  }
+  CU(cudaMemcpyAsync(c->d_cs.as<unsigned char>(), c->h_cs.as<unsigned char>(), K, cudaMemcpyHostToDevice, c->stream));
+  return LANDING_OK;
+}
+
+// One buffer argument of a batched call: `bytes` at the caller's input `in` or output `out` (both NULL: absent).
+// `dev` is what the kernels read or write (stage_in); `aos` the caller-layout buffer while they use a transposed copy.
+struct Piece {
+  const void* in;
+  void* out;
+  size_t bytes;
+  void* dev;
+  void* aos;
+  template <class T>
+  T* at() const { return static_cast<T*>(dev); }
+};
+template <class T>
+static Piece input(const T* p, long long n) { return {p, nullptr, sizeof(T) * n, nullptr, nullptr}; }
+template <class T>
+static Piece output(T* p, long long n) { return {nullptr, p, sizeof(T) * n, nullptr, nullptr}; }
+static size_t padded(size_t bytes) { return (bytes + 7) & ~(size_t)7; }
+static size_t staged_bytes(const Piece* pc, int n) {
+  size_t tot = 256;
+  for (int i = 0; i < n; i++)
+    if (pc[i].in || pc[i].out) tot += padded(pc[i].bytes);
+  return tot;
+}
+
+// Host buffers of a batched call.  LANDING_DEVICE: the kernels use the caller's pointers.  LANDING_HOST: the present
+// pieces are laid out in the context's grow-only staging buffer and the inputs copied in (cudaMemcpyAsync on the
+// context's stream); stage_out() copies the outputs back and synchronises the stream once.
+// zero_copy (small host calls -- the CasADi ABI's one scenario per call above all): the pieces go to a mapped pinned
+// buffer instead, the CPU copies the inputs in, the kernels read them and write their results through the device alias
+// of that buffer, and the CPU copies the results out after the stream synchronisation: one launch + one synchronisation
+// per call instead of up to a dozen pageable cudaMemcpyAsync.  Not for kernels that accumulate with device-scope atomics
+// (nlp_grad's parameter sensitivities).
+static int stage_in(landing_ctx* c, int memspace, Piece* pc, int n, bool zero_copy = false) {
+  if (memspace != LANDING_HOST) {
+    for (int i = 0; i < n; i++) pc[i].dev = pc[i].in ? const_cast<void*>(pc[i].in) : pc[i].out;
+    return LANDING_OK;
+  }
+  if (zero_copy) CU(c->pin.reserve(staged_bytes(pc, n)));
+  else CU(c->stage.reserve(staged_bytes(pc, n)));
+  char* cur = zero_copy ? c->pin.as<char>() : c->stage.as<char>();
+  for (int i = 0; i < n; i++) {
+    pc[i].dev = nullptr;
+    if (!pc[i].in && !pc[i].out) continue;
+    pc[i].dev = cur;
+    if (pc[i].in && zero_copy) std::memcpy(cur, pc[i].in, pc[i].bytes);
+    else if (pc[i].in) CU(cudaMemcpyAsync(cur, pc[i].in, pc[i].bytes, cudaMemcpyHostToDevice, c->stream));
+    cur += padded(pc[i].bytes);
+  }
+  return LANDING_OK;
+}
+static int stage_out(landing_ctx* c, int memspace, const Piece* pc, int n, bool zero_copy = false) {
+  if (memspace != LANDING_HOST) return LANDING_OK;
+  if (zero_copy) CU(cudaStreamSynchronize(c->stream));
+  for (int i = 0; i < n; i++) {
+    if (!pc[i].out) continue;
+    if (zero_copy) std::memcpy(pc[i].out, pc[i].dev, pc[i].bytes);
+    else CU(cudaMemcpyAsync(pc[i].out, pc[i].dev, pc[i].bytes, cudaMemcpyDeviceToHost, c->stream));
+  }
+  if (!zero_copy) CU(cudaStreamSynchronize(c->stream));
+  return LANDING_OK;
+}
+
+// AoS batches (one CasADi vector per scenario) would make every warp access 32 different rows: for batches (B >= 64)
+// the kernels run on transposed (SoA) copies instead and the results are transposed back through shared-memory tiles
+// (3 x the traffic of a SoA call, but coalesced: DESIGN.md 2.2).  Small batches (the CasADi ABI: B = 1) go direct.
+// pc[0..n) are staged [B][n_i] double arrays: the inputs are transposed into the context's scratch, the outputs
+// redirected to it, and *layout becomes LANDING_SOA; soa_to_aos() transposes the outputs back after the launch.
+static int aos_to_soa(landing_ctx* c, long long B, int* layout, Piece* pc, int n) {
+  if (*layout != LANDING_AOS || B < 64) return LANDING_OK;
+  CU(c->tr.reserve(staged_bytes(pc, n)));
+  double* cur = c->tr.as<double>();
+  for (int i = 0; i < n; i++) {
+    if (!pc[i].dev) continue;
+    const long long rows = (long long)(pc[i].bytes / sizeof(double)) / B;
+    if (pc[i].in) c->launches += launch_transpose(pc[i].at<const double>(), cur, B, rows, c->stream);  // [B][n] -> [n][B]
+    pc[i].aos = pc[i].dev;
+    pc[i].dev = cur;
+    cur += rows * B;
+  }
+  *layout = LANDING_SOA;
+  return LANDING_OK;
+}
+static void soa_to_aos(landing_ctx* c, long long B, Piece* pc, int n) {
+  for (int i = 0; i < n; i++)
+    if (pc[i].out && pc[i].aos) {
+      const long long rows = (long long)(pc[i].bytes / sizeof(double)) / B;
+      // [n][B] -> [B][n]
+      c->launches += launch_transpose(pc[i].at<const double>(), static_cast<double*>(pc[i].aos), rows, B, c->stream);
+      pc[i].dev = pc[i].aos;
     }
-    CU(cudaMemcpyAsync(c->d_cs, c->h_cs, K, cudaMemcpyHostToDevice, c->stream));
-  } else if (pb->formulation != 0) {
-    return fail(LANDING_ERR_ARG, "landing_problem: formulation must be 0 or 1");
-  }
-  return LANDING_OK;
-}
-
-static int ensure_tr(landing_ctx* c, size_t bytes) {
-  if (bytes <= c->tr_bytes) return LANDING_OK;
-  if (c->tr) cudaFree(c->tr);
-  c->tr = nullptr;
-  c->tr_bytes = 0;
-  CU(cudaMalloc(&c->tr, bytes));
-  c->tr_bytes = bytes;
-  return LANDING_OK;
-}
-
-static int ensure_pin(landing_ctx* c, size_t bytes) {
-  if (bytes <= c->pin_bytes) return LANDING_OK;
-  if (c->pin) cudaFreeHost(c->pin);
-  c->pin = nullptr;
-  c->pin_bytes = 0;
-  if (bytes < (64u << 10)) bytes = 64u << 10;
-  CU(cudaHostAlloc(&c->pin, bytes, cudaHostAllocMapped));
-  c->pin_bytes = bytes;
-  return LANDING_OK;
-}
-
-static int ensure_stage(landing_ctx* c, size_t bytes) {
-  if (bytes <= c->stage_bytes) return LANDING_OK;
-  if (c->stage) cudaFree(c->stage);
-  c->stage = nullptr;
-  c->stage_bytes = 0;
-  CU(cudaMalloc(&c->stage, bytes));
-  c->stage_bytes = bytes;
-  return LANDING_OK;
 }
 
 extern "C" {
@@ -190,18 +249,12 @@ int landing_create(int N, int device, landing_ctx** out) {
 void landing_destroy(landing_ctx* c) {
   if (!c) return;
   DeviceGuard guard_(c->device);
+  const cudaStream_t st = c->stream;
   solver_free(c->ws);
-  if (c->stage) cudaFree(c->stage);
-  if (c->pin) cudaFreeHost(c->pin);
-  if (c->tr) cudaFree(c->tr);
   if (c->d_maps) cudaFree(c->d_maps);
-  if (c->d_dt) cudaFree(c->d_dt);
-  if (c->h_dt) cudaFreeHost(c->h_dt);
-  if (c->d_cs) cudaFree(c->d_cs);
-  if (c->h_cs) cudaFreeHost(c->h_cs);
   if (c->d_kino) cudaFree(c->d_kino);
-  if (c->stream) cudaStreamDestroy(c->stream);
-  delete c;
+  delete c;  // (the grow-only buffers)
+  if (st) cudaStreamDestroy(st);
 }
 
 int landing_dims(const landing_ctx* c, long long d[6]) {
@@ -266,36 +319,6 @@ void landing_kino_setup_default(landing_kino_setup* k) {
   k->jpos_guess[0] = 0.0; k->jpos_guess[1] = -PI / 4; k->jpos_guess[2] = PI / 2;
 }
 
-// inputs / outputs of the two set-up calls staged through the context's buffer when they live in host memory
-struct KinoBuf { const double* in; double* out; long long n; };
-static int kino_stage(landing_ctx* c, long long B, int memspace, KinoBuf* bufs, int nb, const double** din, double** dout) {
-  size_t tot = 0;
-  for (int i = 0; i < nb; i++) if (bufs[i].in || bufs[i].out) tot += sizeof(double) * bufs[i].n * B;
-  if (memspace != LANDING_HOST) {
-    for (int i = 0; i < nb; i++) { din[i] = bufs[i].in; dout[i] = bufs[i].out; }
-    return LANDING_OK;
-  }
-  int rc = ensure_stage(c, tot + 256);
-  if (rc) return rc;
-  char* s = (char*)c->stage;
-  for (int i = 0; i < nb; i++) {
-    din[i] = nullptr; dout[i] = nullptr;
-    if (!bufs[i].in && !bufs[i].out) continue;
-    const size_t by = sizeof(double) * bufs[i].n * B;
-    if (bufs[i].in) { CU(cudaMemcpyAsync(s, bufs[i].in, by, cudaMemcpyHostToDevice, c->stream)); din[i] = (const double*)s; }
-    else dout[i] = (double*)s;
-    s += by;
-  }
-  return LANDING_OK;
-}
-static int kino_unstage(landing_ctx* c, long long B, int memspace, KinoBuf* bufs, int nb, double** dout) {
-  if (memspace != LANDING_HOST) return LANDING_OK;
-  for (int i = 0; i < nb; i++)
-    if (bufs[i].out) CU(cudaMemcpyAsync(bufs[i].out, dout[i], sizeof(double) * bufs[i].n * B, cudaMemcpyDeviceToHost, c->stream));
-  CU(cudaStreamSynchronize(c->stream));
-  return LANDING_OK;
-}
-
 int landing_kino_setup_batch(landing_ctx* c, long long B, int memspace, int layout, const landing_kino_setup* ks,
                              const double* drops, const double* x_srb, double* lbg, double* ubg, double* x0) {
   if (!c || !ks || !drops || B < 0) return fail(LANDING_ERR_ARG, "landing_kino_setup_batch: bad arguments");
@@ -303,20 +326,20 @@ int landing_kino_setup_batch(landing_ctx* c, long long B, int memspace, int layo
   DeviceGuard guard_(c->device);
   auto pl = get_kino_plan(c->N);
   const long long nsrb = 36LL * c->N - 24;
-  KinoBuf bufs[5] = {{drops, nullptr, 12}, {x_srb, nullptr, nsrb}, {nullptr, lbg, pl->m}, {nullptr, ubg, pl->m}, {nullptr, x0, pl->nx}};
-  const double* din[5]; double* dout[5];
-  int rc = kino_stage(c, B, memspace, bufs, 5, din, dout);
+  Piece pc[5] = {input(drops, 12 * B), input(x_srb, nsrb * B), output(lbg, pl->m * B), output(ubg, pl->m * B),
+                 output(x0, pl->nx * B)};
+  int rc = stage_in(c, memspace, pc, 5);
   if (rc) return rc;
   KinoSetupArgs a{};
   a.N = c->N; a.B = B; a.ks = *ks;
-  a.drops = make_cview(din[0], 12, B, layout);
-  a.x_srb = make_cview(din[1], nsrb, B, layout);
-  a.lbg = make_view(dout[2], pl->m, B, layout);
-  a.ubg = make_view(dout[3], pl->m, B, layout);
-  a.x0 = make_view(dout[4], pl->nx, B, layout);
+  a.drops = make_cview(pc[0].at<const double>(), 12, B, layout);
+  a.x_srb = make_cview(pc[1].at<const double>(), nsrb, B, layout);
+  a.lbg = make_view(pc[2].at<double>(), pl->m, B, layout);
+  a.ubg = make_view(pc[3].at<double>(), pl->m, B, layout);
+  a.x0 = make_view(pc[4].at<double>(), pl->nx, B, layout);
   c->launches += launch_kino_setup(a, c->stream);
   CU(cudaGetLastError());
-  return kino_unstage(c, B, memspace, bufs, 5, dout);
+  return stage_out(c, memspace, pc, 5);
 }
 
 int landing_kino_cost_batch(landing_ctx* c, long long B, int memspace, int layout, const landing_kino_setup* ks,
@@ -325,18 +348,17 @@ int landing_kino_cost_batch(landing_ctx* c, long long B, int memspace, int layou
   if (B == 0 || (!f && !grad_f)) return LANDING_OK;
   DeviceGuard guard_(c->device);
   auto pl = get_kino_plan(c->N);
-  KinoBuf bufs[3] = {{x, nullptr, pl->nx}, {nullptr, f, 1}, {nullptr, grad_f, pl->nx}};
-  const double* din[3]; double* dout[3];
-  int rc = kino_stage(c, B, memspace, bufs, 3, din, dout);
+  Piece pc[3] = {input(x, pl->nx * B), output(f, B), output(grad_f, pl->nx * B)};
+  int rc = stage_in(c, memspace, pc, 3);
   if (rc) return rc;
   KinoSetupArgs a{};
   a.N = c->N; a.B = B; a.ks = *ks;
-  a.x = make_cview(din[0], pl->nx, B, layout);
-  a.f = make_view(dout[1], 1, B, layout);
-  a.grad_f = make_view(dout[2], pl->nx, B, layout);
+  a.x = make_cview(pc[0].at<const double>(), pl->nx, B, layout);
+  a.f = make_view(pc[1].at<double>(), 1, B, layout);
+  a.grad_f = make_view(pc[2].at<double>(), pl->nx, B, layout);
   c->launches += launch_kino_cost(a, c->stream);
   CU(cudaGetLastError());
-  return kino_unstage(c, B, memspace, bufs, 3, dout);
+  return stage_out(c, memspace, pc, 3);
 }
 
 int landing_kino_eval_batch(landing_ctx* c, long long B, int memspace, int layout, const landing_kino_problem* pb,
@@ -353,56 +375,28 @@ int landing_kino_eval_batch(landing_ctx* c, long long B, int memspace, int layou
     c->kino = pl;
   }
   const KinoPlan& pl = *c->kino;
-  // knot spacings through the same staging as the solver's
-  landing_problem tmp{};
-  tmp.dt = pb->dt;
-  int rc = stage_dt(c, &tmp);
+  int rc = stage_dt(c, pb->dt, 0.0);
   if (rc) return rc;
-  const double* dx = x;
-  double *dg = g, *dj = jac;
-  if (memspace == LANDING_HOST) {
-    const size_t bx = sizeof(double) * pl.nx * B, bg = g ? sizeof(double) * pl.m * B : 0, bj = jac ? sizeof(double) * pl.nnz * B : 0;
-    rc = ensure_stage(c, bx + bg + bj + 256);
-    if (rc) return rc;
-    char* s = (char*)c->stage;
-    CU(cudaMemcpyAsync(s, x, bx, cudaMemcpyHostToDevice, c->stream));
-    dx = (const double*)s;
-    dg = g ? (double*)(s + bx) : nullptr;
-    dj = jac ? (double*)(s + bx + bg) : nullptr;
-  }
   // AoS batches (one vector per scenario, what landing_solve_batch / landing_kino_setup_batch hand over) are evaluated
-  // on transposed copies like the SRB functions (landing_eval_batch): three times the traffic, all of it coalesced.
-  double *aos_g = nullptr, *aos_j = nullptr;
-  if (layout == LANDING_AOS && B >= 64) {
-    rc = ensure_tr(c, sizeof(double) * (pl.nx + (dg ? pl.m : 0) + (dj ? pl.nnz : 0)) * B + 256);
-    if (rc) return rc;
-    double* cur = (double*)c->tr;
-    c->launches += launch_transpose(dx, cur, B, pl.nx, c->stream);  // [B][n_x] -> [n_x][B]
-    dx = cur; cur += pl.nx * B;
-    if (dg) { aos_g = dg; dg = cur; cur += pl.m * B; }
-    if (dj) { aos_j = dj; dj = cur; cur += pl.nnz * B; }
-    layout = LANDING_SOA;
-  }
+  // on transposed copies like the SRB functions (landing_eval_batch)
+  Piece pc[3] = {input(x, pl.nx * B), output(g, pl.m * B), output(jac, pl.nnz * B)};
+  rc = stage_in(c, memspace, pc, 3);
+  if (!rc) rc = aos_to_soa(c, B, &layout, pc, 3);
+  if (rc) return rc;
   KinoArgs a{};
   a.N = c->N; a.B = B;
-  a.x = make_cview(dx, pl.nx, B, layout);
-  a.g = make_view(dg, pl.m, B, layout);
-  a.jac = make_view(dj, pl.nnz, B, layout);
+  a.x = make_cview(pc[0].at<const double>(), pl.nx, B, layout);
+  a.g = make_view(pc[1].at<double>(), pl.m, B, layout);
+  a.jac = make_view(pc[2].at<double>(), pl.nnz, B, layout);
   a.pr.mu = pb->mu; a.pr.mass = pb->mass;
   for (int i = 0; i < 3; i++) { a.pr.Ib[i] = pb->Ib[i]; a.pr.Ib_inv[i] = pb->Ib_inv[i]; }
-  a.dtv = c->d_dt;
+  a.dtv = c->d_dt.as<double>();
   a.gpos = c->d_kino; a.bpos = c->d_kino + pl.gpos.size();
-  c->launches += launch_kino(a, dg != nullptr, dj != nullptr, c->stream);
+  c->launches += launch_kino(a, g != nullptr, jac != nullptr, c->stream);
   CU(cudaGetLastError());
-  if (aos_g) { c->launches += launch_transpose(dg, aos_g, pl.m, B, c->stream); dg = aos_g; }    // [m][B] -> [B][m]
-  if (aos_j) { c->launches += launch_transpose(dj, aos_j, pl.nnz, B, c->stream); dj = aos_j; }
+  soa_to_aos(c, B, pc, 3);
   CU(cudaGetLastError());
-  if (memspace == LANDING_HOST) {
-    if (g) CU(cudaMemcpyAsync(g, dg, sizeof(double) * pl.m * B, cudaMemcpyDeviceToHost, c->stream));
-    if (jac) CU(cudaMemcpyAsync(jac, dj, sizeof(double) * pl.nnz * B, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-  }
-  return LANDING_OK;
+  return stage_out(c, memspace, pc, 3);
 }
 
 int landing_fp64_peak(landing_ctx* c, double* tflops) {
@@ -475,109 +469,36 @@ int landing_eval_batch(landing_ctx* c, long long B, int memspace, int layout, co
   DeviceGuard guard_(c->device);
   const DevicePlan& pl = c->dpl;
   const long long nx = pl.nx, np = pl.np, m = pl.m, nj = pl.nnzJ, nh = pl.nnzH;
-  // sizes (doubles) of the 4 inputs and 7 outputs
-  const long long in_n[4] = {nx, np, 1, m};
-  const double* in_p[4] = {io->x, io->p, io->lam_f, io->lam_g};
-  const long long out_n[7] = {1, m, nx, nj, nh, nx, np};
-  double* out_p[7] = {io->f, io->g, io->grad_f, io->jac, io->hess, io->grad_x, io->grad_p};
-  const double* din[4];
-  double* dout[7];
-  int* dstatus = io->status;
-  // Small host calls -- the CasADi ABI's one scenario per call above all -- go ZERO-COPY: inputs are copied by the CPU
-  // into a mapped pinned buffer, the kernels read them and write their results through the device alias of that buffer,
-  // and the CPU copies the results out after the stream synchronisation.  One launch + one synchronisation per call
-  // instead of up to eleven pageable cudaMemcpyAsync (LANDING_NO_ZEROCOPY=1 restores the staged copies).
-  bool zero_copy = false;
-  if (memspace == LANDING_HOST) {
-    size_t tot = 0;
-    for (int i = 0; i < 4; i++) if (in_p[i]) tot += sizeof(double) * in_n[i] * B;
-    for (int i = 0; i < 7; i++) if (out_p[i]) tot += sizeof(double) * out_n[i] * B;
-    tot += sizeof(int) * B + 256;
-    static const bool no_zc = getenv("LANDING_NO_ZEROCOPY") != nullptr;
-    // (not for nlp_grad: its parameter sensitivities are accumulated with device-scope atomics)
-    zero_copy = !no_zc && tot <= (512u << 10) && B < 64 && !io->grad_x && !io->grad_p;
-    int rc = zero_copy ? ensure_pin(c, tot) : ensure_stage(c, tot);
-    if (rc) return rc;
-    char* cur = (char*)(zero_copy ? c->pin : c->stage);
-    for (int i = 0; i < 4; i++) {
-      din[i] = nullptr;
-      if (in_p[i]) {
-        din[i] = (const double*)cur;
-        if (zero_copy) std::memcpy(cur, in_p[i], sizeof(double) * in_n[i] * B);
-        else CU(cudaMemcpyAsync(cur, in_p[i], sizeof(double) * in_n[i] * B, cudaMemcpyHostToDevice, c->stream));
-        cur += sizeof(double) * in_n[i] * B;
-      }
-    }
-    for (int i = 0; i < 7; i++) {
-      dout[i] = nullptr;
-      if (out_p[i]) { dout[i] = (double*)cur; cur += sizeof(double) * out_n[i] * B; }
-    }
-    dstatus = io->status ? (int*)cur : nullptr;
-  } else {
-    for (int i = 0; i < 4; i++) din[i] = in_p[i];
-    for (int i = 0; i < 7; i++) dout[i] = out_p[i];
-  }
-  // AoS batches (one CasADi vector per scenario) would make every warp access 32 different rows: for batches the
-  // kernels run on transposed (SoA) copies instead and the results are transposed back through shared-memory tiles
-  // (3 x the traffic of a SoA call, but coalesced: DESIGN.md 2.2).  Small batches (the CasADi ABI: B = 1) go direct.
-  double* aos_out[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-  const bool via_soa = (layout == LANDING_AOS && B >= 64);
-  if (via_soa) {
-    size_t tot = 0;
-    for (int i = 0; i < 4; i++) if (din[i]) tot += sizeof(double) * in_n[i] * B;
-    for (int i = 0; i < 7; i++) if (dout[i]) tot += sizeof(double) * out_n[i] * B;
-    int rc = ensure_tr(c, tot + 256);
-    if (rc) return rc;
-    double* cur = (double*)c->tr;
-    for (int i = 0; i < 4; i++)
-      if (din[i]) {
-        c->launches += launch_transpose(din[i], cur, B, in_n[i], c->stream);  // [B][n] -> [n][B]
-        din[i] = cur;
-        cur += in_n[i] * B;
-      }
-    for (int i = 0; i < 7; i++)
-      if (dout[i]) { aos_out[i] = dout[i]; dout[i] = cur; cur += out_n[i] * B; }
-    layout = LANDING_SOA;
-  }
+  Piece pc[12] = {input(io->x, nx * B), input(io->p, np * B), input(io->lam_f, B), input(io->lam_g, m * B),
+                  output(io->f, B), output(io->g, m * B), output(io->grad_f, nx * B), output(io->jac, nj * B),
+                  output(io->hess, nh * B), output(io->grad_x, nx * B), output(io->grad_p, np * B),
+                  output(io->status, B)};
+  static const bool no_zc = getenv("LANDING_NO_ZEROCOPY") != nullptr;  // restores the staged copies
+  const bool zero_copy = memspace == LANDING_HOST && !no_zc && B < 64 && !io->grad_x && !io->grad_p &&
+                         staged_bytes(pc, 12) <= (512u << 10);
+  int rc = stage_in(c, memspace, pc, 12, zero_copy);
+  if (!rc) rc = aos_to_soa(c, B, &layout, pc, 11);  // (status is [B] in both layouts)
+  if (rc) return rc;
   EvalArgs a{};
   a.pl = pl;
   a.B = B;
-  a.x = make_cview(din[0], nx, B, layout);
-  a.p = make_cview(din[1], np, B, layout);
-  a.lam_f = make_cview(din[2], 1, B, layout);
-  a.lam_g = make_cview(din[3], m, B, layout);
-  a.f = make_view(dout[0], 1, B, layout);
-  a.g = make_view(dout[1], m, B, layout);
-  a.grad_f = make_view(dout[2], nx, B, layout);
-  a.jac = make_view(dout[3], nj, B, layout);
-  a.hess = make_view(dout[4], nh, B, layout);
-  a.grad_x = make_view(dout[5], nx, B, layout);
-  a.grad_p = make_view(dout[6], np, B, layout);
-  a.status = dstatus;
+  a.x = make_cview(pc[0].at<const double>(), nx, B, layout);
+  a.p = make_cview(pc[1].at<const double>(), np, B, layout);
+  a.lam_f = make_cview(pc[2].at<const double>(), 1, B, layout);
+  a.lam_g = make_cview(pc[3].at<const double>(), m, B, layout);
+  a.f = make_view(pc[4].at<double>(), 1, B, layout);
+  a.g = make_view(pc[5].at<double>(), m, B, layout);
+  a.grad_f = make_view(pc[6].at<double>(), nx, B, layout);
+  a.jac = make_view(pc[7].at<double>(), nj, B, layout);
+  a.hess = make_view(pc[8].at<double>(), nh, B, layout);
+  a.grad_x = make_view(pc[9].at<double>(), nx, B, layout);
+  a.grad_p = make_view(pc[10].at<double>(), np, B, layout);
+  a.status = pc[11].at<int>();
   c->launches += launch_eval(a, c->stream);
   CU(cudaGetLastError());
-  if (via_soa) {
-    for (int i = 0; i < 7; i++)
-      if (aos_out[i]) {
-        c->launches += launch_transpose(dout[i], aos_out[i], out_n[i], B, c->stream);  // [n][B] -> [B][n]
-        dout[i] = aos_out[i];
-      }
-    CU(cudaGetLastError());
-  }
-  if (memspace == LANDING_HOST && zero_copy) {
-    CU(cudaStreamSynchronize(c->stream));
-    for (int i = 0; i < 7; i++)
-      if (out_p[i]) std::memcpy(out_p[i], dout[i], sizeof(double) * out_n[i] * B);
-    if (io->status) std::memcpy(io->status, dstatus, sizeof(int) * B);
-  } else if (memspace == LANDING_HOST) {
-    for (int i = 0; i < 7; i++)
-      if (out_p[i])
-        CU(cudaMemcpyAsync(out_p[i], dout[i], sizeof(double) * out_n[i] * B, cudaMemcpyDeviceToHost, c->stream));
-    if (io->status)
-      CU(cudaMemcpyAsync(io->status, dstatus, sizeof(int) * B, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-  }
-  return LANDING_OK;
+  soa_to_aos(c, B, pc, 11);
+  CU(cudaGetLastError());
+  return stage_out(c, memspace, pc, 12, zero_copy);
 }
 
 void landing_tvlqr_default(landing_tvlqr* q) {
@@ -602,27 +523,15 @@ int landing_tvlqr_batch(landing_ctx* c, long long B, int memspace, const landing
   if (B == 0) return LANDING_OK;
   DeviceGuard guard_(c->device);
   const long long nx = c->dpl.nx, ns = par->n_steps;
+  Piece pc[3] = {input(x_star, nx * B), output(P_out, 576 * ns * B), output(K_out, 288 * ns * B)};
+  int rc = stage_in(c, memspace, pc, 3);
+  if (rc) return rc;
   TvlqrArgs a{};
   a.N = c->N; a.nx = nx; a.par = *par;
-  a.x_star = x_star; a.P_out = P_out; a.K_out = K_out;
-  if (memspace == LANDING_HOST) {
-    const size_t bx = sizeof(double) * nx * B, bp = P_out ? sizeof(double) * 576 * ns * B : 0, bk = K_out ? sizeof(double) * 288 * ns * B : 0;
-    int rc = ensure_stage(c, bx + bp + bk + 256);
-    if (rc) return rc;
-    char* s = (char*)c->stage;
-    CU(cudaMemcpyAsync(s, x_star, bx, cudaMemcpyHostToDevice, c->stream));
-    a.x_star = (const double*)s;
-    a.P_out = P_out ? (double*)(s + bx) : nullptr;
-    a.K_out = K_out ? (double*)(s + bx + bp) : nullptr;
-  }
+  a.x_star = pc[0].at<const double>(); a.P_out = pc[1].at<double>(); a.K_out = pc[2].at<double>();
   c->launches += launch_tvlqr(a, B, c->stream);
   CU(cudaGetLastError());
-  if (memspace == LANDING_HOST) {
-    if (P_out) CU(cudaMemcpyAsync(P_out, a.P_out, sizeof(double) * 576 * ns * B, cudaMemcpyDeviceToHost, c->stream));
-    if (K_out) CU(cudaMemcpyAsync(K_out, a.K_out, sizeof(double) * 288 * ns * B, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-  }
-  return LANDING_OK;
+  return stage_out(c, memspace, pc, 3);
 }
 
 int landing_bounds_batch(landing_ctx* c, long long B, int memspace, int layout, const double* p,
@@ -630,26 +539,14 @@ int landing_bounds_batch(landing_ctx* c, long long B, int memspace, int layout, 
   if (!c || !p || !lbg || !ubg || B <= 0) return fail(LANDING_ERR_ARG, "landing_bounds_batch: bad arguments");
   DeviceGuard guard_(c->device);
   const DevicePlan& pl = c->dpl;
-  const double* dp = p;
-  double *dl = lbg, *du = ubg;
-  if (memspace == LANDING_HOST) {
-    int rc = ensure_stage(c, sizeof(double) * B * (pl.np + 2LL * pl.m));
-    if (rc) return rc;
-    double* s = (double*)c->stage;
-    CU(cudaMemcpyAsync(s, p, sizeof(double) * B * pl.np, cudaMemcpyHostToDevice, c->stream));
-    dp = s;
-    dl = s + B * pl.np;
-    du = dl + B * pl.m;
-  }
-  c->launches += launch_bounds(pl, B, make_cview(dp, pl.np, B, layout), make_view(dl, pl.m, B, layout),
-                               make_view(du, pl.m, B, layout), c->stream);
+  Piece pc[3] = {input(p, pl.np * B), output(lbg, pl.m * B), output(ubg, pl.m * B)};
+  int rc = stage_in(c, memspace, pc, 3);
+  if (rc) return rc;
+  c->launches += launch_bounds(pl, B, make_cview(pc[0].at<const double>(), pl.np, B, layout),
+                               make_view(pc[1].at<double>(), pl.m, B, layout), make_view(pc[2].at<double>(), pl.m, B, layout),
+                               c->stream);
   CU(cudaGetLastError());
-  if (memspace == LANDING_HOST) {
-    CU(cudaMemcpyAsync(lbg, dl, sizeof(double) * B * pl.m, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaMemcpyAsync(ubg, du, sizeof(double) * B * pl.m, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-  }
-  return LANDING_OK;
+  return stage_out(c, memspace, pc, 3);
 }
 
 int landing_build_batch(landing_ctx* c, long long B, int memspace, int layout, const landing_problem* pb,
@@ -657,30 +554,16 @@ int landing_build_batch(landing_ctx* c, long long B, int memspace, int layout, c
   if (!c || !pb || !drops || B <= 0) return fail(LANDING_ERR_ARG, "landing_build_batch: bad arguments");
   DeviceGuard guard_(c->device);
   const DevicePlan& pl = c->dpl;
-  const double* dd = drops;
-  double *dp = p, *dx = x0;
-  if (memspace == LANDING_HOST) {
-    int rc = ensure_stage(c, sizeof(double) * B * (12 + pl.np + pl.nx));
-    if (rc) return rc;
-    double* s = (double*)c->stage;
-    CU(cudaMemcpyAsync(s, drops, sizeof(double) * B * 12, cudaMemcpyHostToDevice, c->stream));
-    dd = s;
-    dp = p ? s + 12 * B : nullptr;
-    dx = x0 ? s + 12 * B + B * pl.np : nullptr;
-  }
-  {
-    const int rc = stage_dt(c, pb);
-    if (rc) return rc;
-  }
-  c->launches += launch_build(pl, B, *pb, c->d_dt, dd, make_view(dp, pl.np, B, layout), make_view(dx, pl.nx, B, layout),
+  Piece pc[3] = {input(drops, 12 * B), output(p, pl.np * B), output(x0, pl.nx * B)};
+  int rc = stage_in(c, memspace, pc, 3);
+  if (!rc) rc = stage_dt(c, pb->dt, pb->T);
+  if (!rc) rc = stage_cs(c, pb);
+  if (rc) return rc;
+  c->launches += launch_build(pl, B, *pb, c->d_dt.as<double>(), pc[0].at<const double>(),
+                              make_view(pc[1].at<double>(), pl.np, B, layout), make_view(pc[2].at<double>(), pl.nx, B, layout),
                               c->stream);
   CU(cudaGetLastError());
-  if (memspace == LANDING_HOST) {
-    if (p) CU(cudaMemcpyAsync(p, dp, sizeof(double) * B * pl.np, cudaMemcpyDeviceToHost, c->stream));
-    if (x0) CU(cudaMemcpyAsync(x0, dx, sizeof(double) * B * pl.nx, cudaMemcpyDeviceToHost, c->stream));
-    CU(cudaStreamSynchronize(c->stream));
-  }
-  return LANDING_OK;
+  return stage_out(c, memspace, pc, 3);
 }
 
 int landing_solve_batch(landing_ctx* c, long long B, int memspace, const landing_problem* pb,
@@ -691,34 +574,37 @@ int landing_solve_batch(landing_ctx* c, long long B, int memspace, const landing
   DeviceGuard guard_(c->device);
   landing_options o;
   if (opt) o = *opt; else landing_options_default(&o);
+  int rc = stage_dt(c, pb->dt, pb->T);
+  if (!rc) rc = stage_cs(c, pb);
+  if (rc) return rc;
+  const long long nx = c->dpl.nx, m = c->dpl.m;
+  Piece pc[8] = {input(io->drops, 12 * B), input(io->x0, nx * B), output(io->x_star, nx * B), output(io->f_star, B),
+                 output(io->lam_g, m * B), output(io->viol, B), output(io->status, B), output(io->iters, B)};
+  rc = stage_in(c, memspace, pc, 8);
+  if (rc) return rc;
+  const landing_solve_io dio{pc[0].at<const double>(), pc[1].at<const double>(), pc[2].at<double>(), pc[3].at<double>(),
+                             pc[4].at<double>(), pc[5].at<double>(), pc[6].at<int>(), pc[7].at<int>()};
   std::string err;
   int launches = 0;
-  int rc = stage_dt(c, pb);
-  if (rc) return rc;
-  rc = solver_run(c->ws, c->dpl, B, memspace, *pb, c->d_dt, pb->formulation == 1 ? c->d_cs : nullptr, o, *io, c->stream,
-                  &launches, &err);
+  rc = solver_run(c->ws, c->dpl, B, *pb, c->d_dt.as<double>(), pb->formulation == 1 ? c->d_cs.as<unsigned char>() : nullptr,
+                  o, dio, c->stream, &launches, &err);
   c->launches += launches;
   if (rc) return fail(rc, err);
-  return LANDING_OK;
+  return stage_out(c, memspace, pc, 8);
 }
 
 // ---------------------------------------------------------------- several GPUs, one process
 struct landing_multi {
   int N = 0;
   std::vector<landing_ctx*> ctx;
-  struct Shard {  // pinned host staging of one device's shard (grow-only)
-    long long cap = 0, cap_lam = 0, cap_x0 = 0;
-    double *drops = nullptr, *x = nullptr, *f = nullptr, *viol = nullptr, *lam = nullptr, *x0 = nullptr;
-    int *status = nullptr, *iters = nullptr;
-  };
-  std::vector<Shard> sh;
+  std::vector<PinnedBuf> sh;  // pinned host staging of each device's shard
 };
 
 int landing_multi_create(int N, int n_devices, const int* devices, landing_multi** out) {
   if (!out || !devices || n_devices < 1) return fail(LANDING_ERR_ARG, "landing_multi_create: bad arguments");
   std::unique_ptr<landing_multi> m(new landing_multi());
   m->N = N;
-  m->sh.resize(n_devices);
+  m->sh = std::vector<PinnedBuf>(n_devices);
   for (int d = 0; d < n_devices; d++) {
     landing_ctx* c = nullptr;
     const int rc = landing_create(N, devices[d], &c);
@@ -736,9 +622,7 @@ void landing_multi_destroy(landing_multi* m) {
   if (!m) return;
   for (size_t d = 0; d < m->ctx.size(); d++) {
     DeviceGuard guard_(m->ctx[d]->device);
-    landing_multi::Shard& s = m->sh[d];
-    for (void* p : {(void*)s.drops, (void*)s.x, (void*)s.f, (void*)s.viol, (void*)s.lam, (void*)s.x0, (void*)s.status, (void*)s.iters})
-      if (p) cudaFreeHost(p);
+    m->sh[d].release();
     landing_destroy(m->ctx[d]);
   }
   delete m;
@@ -756,43 +640,41 @@ int landing_solve_batch_multi(landing_multi* m, long long B, const landing_probl
   std::vector<std::string> errs(G);
   auto work = [&](int d) {
     landing_ctx* c = m->ctx[d];
-    landing_multi::Shard& s = m->sh[d];
     const long long Bd = (B - d + G - 1) / G;  // scenarios d, d + G, ...
     if (Bd <= 0) return;
     DeviceGuard guard_(c->device);
-    auto grow = [&](auto*& p, long long n) {
-      if (p) cudaFreeHost(p);
-      p = nullptr;
-      return cudaMallocHost((void**)&p, sizeof(*p) * (size_t)n) == cudaSuccess;
-    };
-    bool ok = true;
-    if (Bd > s.cap) {
-      ok = grow(s.drops, 12 * Bd) && grow(s.x, nx * Bd) && grow(s.f, Bd) && grow(s.viol, Bd) && grow(s.status, Bd) &&
-           grow(s.iters, Bd);
-      s.cap = ok ? Bd : 0;
-    }
-    if (ok && io->lam_g && Bd > s.cap_lam) { ok = grow(s.lam, mr * Bd); s.cap_lam = ok ? Bd : 0; }
-    if (ok && io->x0 && Bd > s.cap_x0) { ok = grow(s.x0, nx * Bd); s.cap_x0 = ok ? Bd : 0; }
-    if (!ok) { rcs[d] = LANDING_ERR_CUDA; errs[d] = "landing_solve_batch_multi: pinned host allocation failed"; return; }
-    for (long long i = 0; i < Bd; i++) {
-      const long long b = d + i * G;
-      std::memcpy(s.drops + 12 * i, io->drops + 12 * b, sizeof(double) * 12);
-      if (io->x0) std::memcpy(s.x0 + nx * i, io->x0 + nx * b, sizeof(double) * nx);
+    const long long nd = (12 + nx + 2 + (io->lam_g ? mr : 0) + (io->x0 ? nx : 0)) * Bd;  // doubles, then 2 Bd ints
+    if (m->sh[d].reserve(sizeof(double) * nd + sizeof(int) * 2 * Bd) != cudaSuccess) {
+      rcs[d] = LANDING_ERR_CUDA;
+      errs[d] = "landing_solve_batch_multi: pinned host allocation failed";
+      return;
     }
     landing_solve_io sio{};
-    sio.drops = s.drops; sio.x0 = io->x0 ? s.x0 : nullptr;
-    sio.x_star = s.x; sio.f_star = s.f; sio.lam_g = io->lam_g ? s.lam : nullptr; sio.viol = s.viol;
-    sio.status = s.status; sio.iters = s.iters;
+    double* p = m->sh[d].as<double>();
+    double* drops = p; p += 12 * Bd;
+    sio.x_star = p; p += nx * Bd;
+    sio.f_star = p; p += Bd;
+    sio.viol = p; p += Bd;
+    if (io->lam_g) { sio.lam_g = p; p += mr * Bd; }
+    double* x0 = io->x0 ? p : nullptr; p += io->x0 ? nx * Bd : 0;
+    sio.status = (int*)p;
+    sio.iters = sio.status + Bd;
+    for (long long i = 0; i < Bd; i++) {
+      const long long b = d + i * G;
+      std::memcpy(drops + 12 * i, io->drops + 12 * b, sizeof(double) * 12);
+      if (x0) std::memcpy(x0 + nx * i, io->x0 + nx * b, sizeof(double) * nx);
+    }
+    sio.drops = drops; sio.x0 = x0;
     rcs[d] = landing_solve_batch(c, Bd, LANDING_HOST, pb, opt, &sio);
     if (rcs[d]) { errs[d] = landing_last_error(); return; }
     for (long long i = 0; i < Bd; i++) {  // gather: this device's records into the whole sweep's arrays
       const long long b = d + i * G;
-      std::memcpy(io->x_star + nx * b, s.x + nx * i, sizeof(double) * nx);
-      io->f_star[b] = s.f[i];
-      io->status[b] = s.status[i];
-      io->iters[b] = s.iters[i];
-      if (io->viol) io->viol[b] = s.viol[i];
-      if (io->lam_g) std::memcpy(io->lam_g + mr * b, s.lam + mr * i, sizeof(double) * mr);
+      std::memcpy(io->x_star + nx * b, sio.x_star + nx * i, sizeof(double) * nx);
+      io->f_star[b] = sio.f_star[i];
+      io->status[b] = sio.status[i];
+      io->iters[b] = sio.iters[i];
+      if (io->viol) io->viol[b] = sio.viol[i];
+      if (io->lam_g) std::memcpy(io->lam_g + mr * b, sio.lam_g + mr * i, sizeof(double) * mr);
     }
   };
   std::vector<std::thread> th;

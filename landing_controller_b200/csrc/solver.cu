@@ -290,17 +290,18 @@ int fp64_peak_run(cudaStream_t st, double* tflops, std::string* err) {
 }
 
 void solver_free(SolverWorkspace& ws) {
-  if (ws.scratch) cudaFree(ws.scratch);
-  if (ws.io) cudaFree(ws.io);
   if (ws.counter) cudaFree(ws.counter);
   if (ws.zeros) cudaFree(ws.zeros);
-  if (ws.order) cudaFree(ws.order);
   if (ws.kt) cudaFree(ws.kt);
   if (ws.tab.dev) cudaFree(ws.tab.dev);
-  ws = SolverWorkspace{};
+  ws.counter = nullptr;
+  ws.zeros = nullptr;
+  ws.kt = nullptr;
+  ws.tab = SolverTables{};
+  ws.ready = false;
 }
 
-int solver_run(SolverWorkspace& ws, const DevicePlan& pl, long long B, int memspace,
+int solver_run(SolverWorkspace& ws, const DevicePlan& pl, long long B,
                const landing_problem& pb, const double* dtv, const unsigned char* csm, const landing_options& opt,
                const landing_solve_io& io, cudaStream_t st, int* launches, std::string* err) {
   const int N = pl.N;
@@ -338,15 +339,8 @@ int solver_run(SolverWorkspace& ws, const DevicePlan& pl, long long B, int memsp
   }
   const long long slot = slot_doubles(N);
   const long long nslots = (long long)ws.n_sm * CTAS_PER_SM;
-  const size_t need = sizeof(double) * slot * nslots;
-  if (need > ws.scratch_bytes) {
-    if (ws.scratch) cudaFree(ws.scratch);
-    ws.scratch = nullptr;
-    ws.scratch_bytes = 0;
-    CUS(cudaMalloc(&ws.scratch, need));
-    ws.scratch_bytes = need;
-  }
-  const long long nx = pl.nx, m = pl.m;
+  CUS(ws.scratch.reserve(sizeof(double) * slot * nslots));
+  const long long m = pl.m;
   KParams P{};
   P.N = N; P.K = N - 1; P.nx = pl.nx; P.MR = 36 + RK * (N - 1);
   P.B = B; P.pb = pb; P.pb.dt = nullptr; P.pb.cs = nullptr; P.dtv = dtv; P.csm = csm; P.opt = opt;
@@ -354,34 +348,9 @@ int solver_run(SolverWorkspace& ws, const DevicePlan& pl, long long B, int memsp
   for (int i = 0; i < 12; i++) P.run_qx |= (pb.QX[i] != 0.0);
   P.opt.reserved[0] = pl.m;  // m, for the dual scaling s_d
   P.zeros = ws.zeros;
-  P.counter = ws.counter; P.scratch = ws.scratch; P.slot = slot; P.tab = ws.tab; P.kt = ws.kt;
-  if (memspace == LANDING_HOST) {
-    size_t bytes = sizeof(double) * B * (12 + nx + 2 + (io.x0 ? nx : 0) + (io.lam_g ? m : 0)) + sizeof(int) * 2 * B + 64;
-    if (bytes > ws.io_bytes) {
-      if (ws.io) cudaFree(ws.io);
-      ws.io = nullptr;
-      ws.io_bytes = 0;
-      CUS(cudaMalloc(&ws.io, bytes));
-      ws.io_bytes = bytes;
-    }
-    double* p = (double*)ws.io;
-    double* d_drops = p; p += 12 * B;
-    P.x_star = p; p += nx * B;
-    P.f_star = p; p += B;
-    P.viol = p; p += B;
-    double* d_x0 = nullptr;
-    if (io.x0) { d_x0 = p; p += nx * B; }
-    if (io.lam_g) { P.lam_g = p; p += m * B; }
-    P.status = (int*)p;
-    P.iters = P.status + B;
-    CUS(cudaMemcpyAsync(d_drops, io.drops, sizeof(double) * 12 * B, cudaMemcpyHostToDevice, st));
-    if (io.x0) CUS(cudaMemcpyAsync(d_x0, io.x0, sizeof(double) * nx * B, cudaMemcpyHostToDevice, st));
-    P.drops = d_drops;
-    P.x0 = d_x0;
-  } else {
-    P.drops = io.drops; P.x0 = io.x0; P.x_star = io.x_star; P.f_star = io.f_star; P.lam_g = io.lam_g;
-    P.viol = io.viol; P.status = io.status; P.iters = io.iters;
-  }
+  P.counter = ws.counter; P.scratch = ws.scratch.as<double>(); P.slot = slot; P.tab = ws.tab; P.kt = ws.kt;
+  P.drops = io.drops; P.x0 = io.x0; P.x_star = io.x_star; P.f_star = io.f_star; P.lam_g = io.lam_g;
+  P.viol = io.viol; P.status = io.status; P.iters = io.iters;
 #ifdef SRB_PROF
   static const bool want_prof = getenv("LANDING_PROF") != nullptr;
 #else
@@ -401,28 +370,22 @@ int solver_run(SolverWorkspace& ws, const DevicePlan& pl, long long B, int memsp
     if (by_sort)
       CUS(cub::DeviceRadixSort::SortPairsDescending(nullptr, sort_bytes, (const double*)nullptr, (double*)nullptr,
                                                     (const int*)nullptr, (int*)nullptr, (int)B, 0, 64, st));
-    const size_t need_o = sizeof(int) * B + (by_sort ? (sizeof(double) * 2 + sizeof(int)) * B + sort_bytes + 512 : 0);
-    if (need_o > ws.order_cap) {
-      if (ws.order) cudaFree(ws.order);
-      ws.order = nullptr;
-      ws.order_cap = 0;
-      CUS(cudaMalloc(&ws.order, need_o));
-      ws.order_cap = need_o;
-    }
+    CUS(ws.order.reserve(sizeof(int) * B + (by_sort ? (sizeof(double) * 2 + sizeof(int)) * B + sort_bytes + 512 : 0)));
+    int* order = ws.order.as<int>();
     if (by_sort) {
-      char* base = reinterpret_cast<char*>(ws.order) + ((sizeof(int) * B + 255) / 256) * 256;
+      char* base = reinterpret_cast<char*>(order) + ((sizeof(int) * B + 255) / 256) * 256;
       double* k_in = reinterpret_cast<double*>(base);
       double* k_out = k_in + B;
       int* id_in = reinterpret_cast<int*>(k_out + B);
       void* tmp = reinterpret_cast<char*>(id_in) + ((sizeof(int) * B + 255) / 256) * 256;
       k_order_keys<<<(unsigned)((B + 255) / 256), 256, 0, st>>>(P.drops, B, k_in, id_in);
-      CUS(cub::DeviceRadixSort::SortPairsDescending(tmp, sort_bytes, k_in, k_out, id_in, ws.order, (int)B, 0, 64, st));
+      CUS(cub::DeviceRadixSort::SortPairsDescending(tmp, sort_bytes, k_in, k_out, id_in, order, (int)B, 0, 64, st));
       *launches += 2;
     } else {
-      k_order<<<(unsigned)((B + 255) / 256), 256, 0, st>>>(P.drops, B, ws.order);
+      k_order<<<(unsigned)((B + 255) / 256), 256, 0, st>>>(P.drops, B, order);
       *launches += 1;
     }
-    P.order = ws.order;
+    P.order = order;
   }
   if (P.lam_g) CUS(cudaMemsetAsync(P.lam_g, 0, sizeof(double) * m * B, st));
   long long gcap = nslots;
@@ -458,15 +421,6 @@ int solver_run(SolverWorkspace& ws, const DevicePlan& pl, long long B, int memsp
       if (h[PH_X0 + i]) fprintf(stderr, "[landing prof]   X%d %10.0f cycles per iteration\n", i, (double)h[PH_X0 + i] / (double)std::max(1ull, h[PH_NITER]));
     fprintf(stderr, "[landing prof]   one lap of the instrumentation costs %.0f cycles\n",
             (double)h[PH_CAL] / (4.0 * (double)std::max(1ull, h[PH_NITER])));
-  }
-  if (memspace == LANDING_HOST) {
-    CUS(cudaMemcpyAsync(io.x_star, P.x_star, sizeof(double) * nx * B, cudaMemcpyDeviceToHost, st));
-    CUS(cudaMemcpyAsync(io.f_star, P.f_star, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
-    if (io.viol) CUS(cudaMemcpyAsync(io.viol, P.viol, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
-    if (io.lam_g) CUS(cudaMemcpyAsync(io.lam_g, P.lam_g, sizeof(double) * m * B, cudaMemcpyDeviceToHost, st));
-    CUS(cudaMemcpyAsync(io.status, P.status, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
-    CUS(cudaMemcpyAsync(io.iters, P.iters, sizeof(int) * B, cudaMemcpyDeviceToHost, st));
-    CUS(cudaStreamSynchronize(st));
   }
   return LANDING_OK;
 }

@@ -2,6 +2,7 @@
 #pragma once
 #include <string>
 
+#include "growbuf.cuh"
 #include "kernels.cuh"
 
 namespace srb {
@@ -27,26 +28,25 @@ struct SolverTables {
 };
 
 struct SolverWorkspace {
-  double* scratch = nullptr;  // per-warp-slot scratch (iterate, lists, Riccati factors)
-  size_t scratch_bytes = 0;
-  void* io = nullptr;         // staging of drops / results for host-buffer calls
-  size_t io_bytes = 0;
+  DeviceBuf scratch;          // per-warp-slot scratch (iterate, lists, Riccati factors)
   int* counter = nullptr;     // work-queue head
   double* zeros = nullptr;    // 16 zeros (c+ operand of the last knot)
-  int* order = nullptr;       // work-queue order (scenario ids, longest expected first)
+  DeviceBuf order;            // work-queue order (scenario ids, longest expected first), and for large sweeps the
+                              // sort keys / ids / temporary storage behind it
   unsigned char* kt = nullptr;  // row-kind tables (k_kinds)
-  size_t order_cap = 0;       // bytes (order, and for large sweeps the sort keys / ids / temporary storage behind it)
   SolverTables tab;
   int n_sm = 0;
   bool ready = false;         // first-call set-up (tables, queue head, kernel attributes) completed
 };
 
+// frees the first-call set-up (the grow-only buffers free themselves)
 void solver_free(SolverWorkspace& ws);
 
 // FP64 FMA throughput of the device (roofline denominator of the interior-point kernel), TFLOP/s
 int fp64_peak_run(cudaStream_t st, double* tflops, std::string* err);
 
-int solver_run(SolverWorkspace& ws, const DevicePlan& pl, long long B, int memspace,
+// io: device pointers
+int solver_run(SolverWorkspace& ws, const DevicePlan& pl, long long B,
                const landing_problem& pb, const double* dtv, const unsigned char* csm, const landing_options& opt,
                const landing_solve_io& io,
                cudaStream_t st, int* launches, std::string* err);
