@@ -201,7 +201,8 @@ typedef struct landing_tvlqr {
   double T;        /* horizon of the trajectories (knot spacing T/(N-1)) */
   double dt;       /* Riccati step, 0.022 in the reference */
   int n_steps;     /* time points */
-  double Q[576], F[576], R[12]; /* running weight, terminal weight, diagonal of the control weight (90) */
+  double Q[576], F[576], R[12]; /* running weight, terminal weight, diagonal of the control weight (90); Q and F must
+                                   be symmetric: P stays symmetric and A'P + PA is formed as W + W' with W = A'P */
   double Ib[9];    /* full 3x3 body inertia, get_mass_matrix(model, zeros(18,1), 0) */
   double mass;
 } landing_tvlqr;

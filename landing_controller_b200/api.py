@@ -371,10 +371,11 @@ class LandingSolver:
         for i in range(3):
             pb.Ib[i] = self.problem.Ib[i] if Ib is None else Ib[i]
             pb.Ib_inv[i] = self.problem.Ib_inv[i] if Ib_inv is None else Ib_inv[i]
-        self._kino_dt = np.ascontiguousarray(dt, dtype=np.float64)
-        if self._kino_dt.shape != (self.N - 1,):
+        dt = np.ascontiguousarray(dt, dtype=np.float64)
+        if dt.shape != (self.N - 1,):
             raise ValueError("dt must have N-1 = %d entries" % (self.N - 1))
-        pb.dt = self._kino_dt.ctypes.data_as(_dp)
+        pb._dt = dt  # keeps the host array alive as long as this problem: the library reads it during each call
+        pb.dt = dt.ctypes.data_as(_dp)
         return pb
 
     def kino_eval_host(self, x, pb, want_g=True, want_jac=True, layout=AOS):

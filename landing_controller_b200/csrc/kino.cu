@@ -99,50 +99,21 @@ __global__ void __launch_bounds__(128, KINO_G_CTAS) k_kino_g(KinoArgs a) {
   }
 }
 
-// Jacobian.  A pass seeds one triple of knot-local inputs (three tangents: r | rpy | omega | v | the
-// joint angles, foot position, force, next foot position of one leg | a triple of the next state) and runs the knot
-// function with that block typed DualN<3> and every other block a plain double, restricted to the row groups the triple
-// can reach; the rpy triple, which reaches every leg's rows through R, is split into five passes (dynamics, four legs).
-constexpr int JAC_PASSES = 28;
-template <int G> struct PassOf {  // pass -> (first seeded input, row groups)
-  static constexpr int v0 = G < 24 ? 3 * G : 3;
-  static constexpr unsigned mask = G == 1 ? kino::G_DYN : G >= 24 ? (kino::G_LEG0 << (G - 24)) : kino::reach(3 * G);
-};
+// Jacobian: the passes of kino_knot.cuh (kino::PassOf, kino::jac_pass), one thread per (scenario, knot, pass).
 template <bool LAST, int G>
 __device__ __forceinline__ void kino_jac_pass(const KinoArgs& a, long long b, int k) {
-  using D = kino::DualN<3>;
-  constexpr int v0 = PassOf<G>::v0, blk = v0 < 12 ? v0 / 3 : v0 < 24 ? 4 : v0 < 36 ? 5 : v0 < 48 ? 6 : v0 < 60 ? 7 : 8;
   double x[NIN];  // (loads of inputs the pass never uses are dead code)
 #pragma unroll
   for (int v = 0; v < NIN; v++) x[v] = (LAST && v >= 60) ? 0.0 : a.x.get(kino_col(a.N, k, v), b);
   const double h = __ldg(a.dtv + k);
-  JSinkN<3> s{a.jac, b, a.gpos + ((long long)k * NIN + v0) * ROWS_INT};
-  constexpr unsigned mask = PassOf<G>::mask;
-  if constexpr (blk < 4) {  // a triple of X_k
-    D t[3];
-#pragma unroll
-    for (int j = 0; j < 3; j++) t[j] = kino::seeded<3>(x[v0 + j], j);
-    if constexpr (blk == 0) kino::knot_rows_h<LAST>(t, x + 3, x + 6, x + 9, x + 12, x + 24, x + 36, x + 48, x + 60, h, a.pr, s, mask);
-    if constexpr (blk == 1) kino::knot_rows_h<LAST>(x, t, x + 6, x + 9, x + 12, x + 24, x + 36, x + 48, x + 60, h, a.pr, s, mask);
-    if constexpr (blk == 2) kino::knot_rows_h<LAST>(x, x + 3, t, x + 9, x + 12, x + 24, x + 36, x + 48, x + 60, h, a.pr, s, mask);
-    if constexpr (blk == 3) kino::knot_rows_h<LAST>(x, x + 3, x + 6, t, x + 12, x + 24, x + 36, x + 48, x + 60, h, a.pr, s, mask);
-  } else {  // a triple of a 12-block: the block as duals, tangents on the triple
-    constexpr int base = 12 * (blk - 3), off = v0 - base;
-    D t[12];
-#pragma unroll
-    for (int i = 0; i < 12; i++) t[i] = (i >= off && i < off + 3) ? kino::seeded<3>(x[base + i], i - off) : D(x[base + i]);
-    if constexpr (blk == 4) kino::knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, t, x + 24, x + 36, x + 48, x + 60, h, a.pr, s, mask);
-    if constexpr (blk == 5) kino::knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, x + 12, t, x + 36, x + 48, x + 60, h, a.pr, s, mask);
-    if constexpr (blk == 6) kino::knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, x + 12, x + 24, t, x + 48, x + 60, h, a.pr, s, mask);
-    if constexpr (blk == 7) kino::knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, x + 12, x + 24, x + 36, t, x + 60, h, a.pr, s, mask);
-    if constexpr (blk == 8) kino::knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, x + 12, x + 24, x + 36, x + 48, t, h, a.pr, s, mask);
-  }
+  JSinkN<3> s{a.jac, b, a.gpos + ((long long)k * NIN + kino::PassOf<G>::v0) * ROWS_INT};
+  kino::jac_pass<LAST, G>(x, h, a.pr, s);
 }
 template <bool LAST, int G, int G1>
 __device__ __forceinline__ void kino_jac_dispatch(const KinoArgs& a, long long b, int k, int g) {
   if constexpr (G < G1) {
     if (g == G) {
-      if constexpr (!(LAST && G >= 20 && G < 24)) kino_jac_pass<LAST, G>(a, b, k);  // (no c_{k+1} in the last knot)
+      if constexpr (kino::pass_in_knot(LAST, G)) kino_jac_pass<LAST, G>(a, b, k);
     } else {
       kino_jac_dispatch<LAST, G + 1, G1>(a, b, k, g);
     }

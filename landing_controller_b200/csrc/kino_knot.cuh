@@ -284,6 +284,46 @@ KHD void knot_rows(const S* in, double h, const Params& pr, bool last, Sink& out
   else knot_rows_t<false, S, Sink>(in, h, pr, out, mask);
 }
 
+// Jacobian passes.  A pass seeds one triple of knot-local inputs (three tangents: r | rpy | omega | v | the
+// joint angles, foot position, force, next foot position of one leg | a triple of the next state) and runs the knot
+// function with that block typed DualN<3> and every other block a plain double, restricted to the row groups the triple
+// can reach; the rpy triple, which reaches every leg's rows through R, is split into five passes (dynamics, four legs).
+// Together the passes emit every non-zero of dg/dz exactly once (tests/test_kino_host.py checks this on the host).
+constexpr int JAC_PASSES = 28;
+template <int G> struct PassOf {  // pass -> (first seeded input, row groups)
+  static constexpr int v0 = G < 24 ? 3 * G : 3;
+  static constexpr unsigned mask = G == 1 ? G_DYN : G >= 24 ? (G_LEG0 << (G - 24)) : reach(3 * G);
+};
+KHD constexpr bool pass_in_knot(bool last, int G) { return !(last && G >= 20 && G < 24); }  // (no c_{k+1} in the last knot)
+
+// Pass G on the knot-local inputs x: out(rho, DualN<3>) gets d row / d x[v0 + j] as tangent j (out(rho, double): a row
+// that does not depend on the triple).
+template <bool LAST, int G, class Sink>
+KHD void jac_pass(const double* x, double h, const Params& pr, Sink& s) {
+  using D = DualN<3>;
+  constexpr int v0 = PassOf<G>::v0, blk = v0 < 12 ? v0 / 3 : v0 < 24 ? 4 : v0 < 36 ? 5 : v0 < 48 ? 6 : v0 < 60 ? 7 : 8;
+  constexpr unsigned mask = PassOf<G>::mask;
+  if constexpr (blk < 4) {  // a triple of X_k
+    D t[3];
+#pragma unroll
+    for (int j = 0; j < 3; j++) t[j] = seeded<3>(x[v0 + j], j);
+    if constexpr (blk == 0) knot_rows_h<LAST>(t, x + 3, x + 6, x + 9, x + 12, x + 24, x + 36, x + 48, x + 60, h, pr, s, mask);
+    if constexpr (blk == 1) knot_rows_h<LAST>(x, t, x + 6, x + 9, x + 12, x + 24, x + 36, x + 48, x + 60, h, pr, s, mask);
+    if constexpr (blk == 2) knot_rows_h<LAST>(x, x + 3, t, x + 9, x + 12, x + 24, x + 36, x + 48, x + 60, h, pr, s, mask);
+    if constexpr (blk == 3) knot_rows_h<LAST>(x, x + 3, x + 6, t, x + 12, x + 24, x + 36, x + 48, x + 60, h, pr, s, mask);
+  } else {  // a triple of a 12-block: the block as duals, tangents on the triple
+    constexpr int base = 12 * (blk - 3), off = v0 - base;
+    D t[12];
+#pragma unroll
+    for (int i = 0; i < 12; i++) t[i] = (i >= off && i < off + 3) ? seeded<3>(x[base + i], i - off) : D(x[base + i]);
+    if constexpr (blk == 4) knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, t, x + 24, x + 36, x + 48, x + 60, h, pr, s, mask);
+    if constexpr (blk == 5) knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, x + 12, t, x + 36, x + 48, x + 60, h, pr, s, mask);
+    if constexpr (blk == 6) knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, x + 12, x + 24, t, x + 48, x + 60, h, pr, s, mask);
+    if constexpr (blk == 7) knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, x + 12, x + 24, x + 36, t, x + 60, h, pr, s, mask);
+    if constexpr (blk == 8) knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, x + 12, x + 24, x + 36, x + 48, t, h, pr, s, mask);
+  }
+}
+
 // Which thread of a (scenario, knot) quadruple owns row rho when the knot is split by leg (k_kino_g): the rows of leg l
 // (contact, hip box, leg length, torques, foot kinematics, joint limits of that leg) belong to part l, everything else
 // (dynamics, f_z, friction, z) to part 0.  constexpr: behind a filtering sink the compiler drops what a part never emits.

@@ -223,13 +223,65 @@ def bounds(pb, q_init, qd_init, c_init):
             ss = [-1, 1, -1, 1][l]
             l_ += [-kx, (-ky if l in (0, 2) else -0.05 * ss), -0.4, -INF]
             u_ += [kx, (-0.05 * ss if l in (0, 2) else ky), -0.075, pb["l_leg_max"] ** 2]
-            l_ += list(-TAU_MAX); u_ += list(TAU_MAX)
+            tau_max = np.asarray(pb.get("tau_max", TAU_MAX))
+            l_ += list(-tau_max); u_ += list(tau_max)
             lb.append(np.array(l_)); ub.append(np.array(u_))
         lb.append(np.full(16, -INF)); ub.append(np.zeros(16))
         lb.append(np.array([pb["z_min"]])); ub.append(np.array([INF]))
         lb += [np.full(12, -0.01), np.full(12, -INF), pb["jpos_min"], np.full(12, -INF)]
         ub += [np.full(12, INF), np.full(12, 0.01), np.full(12, INF), pb["jpos_max"]]
     return np.concatenate(lb), np.concatenate(ub)
+
+
+def knot_col(N, k, v):
+    """Knot-local input v of knot k (X_k 0..11 | jpos_k 12..23 | U_k 24..47 | X_{k+1} 48..59 | c_{k+1} 60..71) -> column
+    of x."""
+    if v < 12: return 12 * k + v
+    if v < 24: return 12 * N + 12 * k + (v - 12)
+    if v < 48: return 24 * N - 12 + 24 * k + (v - 24)
+    if v < 60: return 12 * (k + 1) + (v - 48)
+    return 24 * N - 12 + 24 * (k + 1) + (v - 60)
+
+
+def knot_jac(pb, k, z, last, h=1e-30):
+    """Rows of knot k and their exact Jacobian [rows, len(z)] in the knot-local inputs z (72; 60 for the last knot), by
+    the complex step: d g / d z_j = Im g(z + i h e_j) / h has no subtractive cancellation, so it is exact to rounding.
+    The closed-form kinematics (literal=False) are complex-safe."""
+    z = np.asarray(z, dtype=np.complex128)
+
+    def rows(zz):
+        return knot_rows(pb, k, zz[0:12], zz[48:60], zz[12:24], zz[24:48], None if last else zz[60:72], literal=False)
+
+    J = np.zeros((117 if last else 141, z.size))
+    for j in range(z.size):
+        zz = z.copy()
+        zz[j] += 1j * h
+        J[:, j] = rows(zz).imag / h
+    return rows(z).real, J
+
+
+def jac_exact(pb, x, pattern=None):
+    """Exact dg/dx (tests only): the complex-step Jacobian of every knot (knot_jac) plus the 48 identity entries of the
+    boundary rows.  Dense [m, nx], or with pattern = (colind, row) (CCS) the value array at that pattern."""
+    N = pb["N"]
+    d = dims(N)
+    x = np.asarray(x, dtype=np.float64)
+    Jm = np.zeros((d["m"], d["nx"]))
+    nu = 24 * N - 12  # first column of U
+    bcols = list(range(12)) + [nu + i for i in range(12)] + [12 * (N - 1) + i for i in (0, 1, 2, 3, 4, 5) * 2] + \
+        [12 * (N - 1) + 6 + i for i in (0, 1, 2, 3, 4, 5) * 2]
+    Jm[np.arange(48), bcols] = 1.0
+    for k in range(N - 1):
+        last = k == N - 2
+        cols = [knot_col(N, k, v) for v in range(60 if last else 72)]
+        _, Jk = knot_jac(pb, k, x[cols], last)
+        base = 48 + 141 * k
+        Jm[base:base + Jk.shape[0], cols] = Jk
+    if pattern is None:
+        return Jm
+    colind, row = pattern
+    col = np.repeat(np.arange(d["nx"]), np.diff(colind))
+    return Jm[row, col]
 
 
 def jac_fd(pb, x, h=1e-6, cols=None, literal=True):

@@ -104,3 +104,121 @@ def test_gpu_tvlqr_matches_restatement():
         Pr, Kr = tvlqr_ref.riccati_backward(d["X"][b], U, 0.6, Q, R, F, dt, par.n_steps, z["Ib3"], z["mass"])
         assert np.max(np.abs(P[i] - Pr)) <= 1e-10 * max(1.0, np.abs(Pr).max())
         assert np.max(np.abs(K[i] - Kr)) <= 1e-10 * max(1.0, np.abs(Kr).max())
+
+
+def _spd(rng, n, lo, hi):
+    """Random symmetric positive definite n x n with eigenvalues in [lo, hi], exactly symmetric (the kernel forms
+    A'P + PA as W + W', which needs a symmetric P)."""
+    V, _ = np.linalg.qr(rng.normal(size=(n, n)))
+    S = (V * rng.uniform(lo, hi, n)) @ V.T
+    return 0.5 * (S + S.T)
+
+
+def _weights(rng):
+    """Full (non-diagonal) SPD Q and F over all 24 states, a non-uniform R, a full SPD body inertia with off-diagonal
+    entries and a non-default mass."""
+    z = zero_configuration()
+    Ib = z["Ib3"] + 0.01 * _spd(rng, 3, 0.2, 1.0) + 0.004 * (np.ones((3, 3)) - np.eye(3))
+    return dict(Q=_spd(rng, 24, 0.05, 2.0), F=_spd(rng, 24, 0.5, 6.0), R=rng.uniform(40.0, 150.0, 12), Ib=Ib,
+                mass=rng.uniform(6.0, 11.0))
+
+
+def _random_trajectories(rng, N, B):
+    """Landing-like trajectories X [B, 12, N], U [B, 24, N-1]: feet near their nominal place under the hips, forces up
+    to 100 N per leg."""
+    X = np.empty((B, 12, N))
+    X[:, 0:2], X[:, 2] = rng.uniform(-0.1, 0.1, (B, 2, N)), rng.uniform(0.2, 0.4, (B, N))
+    X[:, 3:6], X[:, 6:12] = rng.uniform(-0.3, 0.3, (B, 3, N)), rng.uniform(-1, 1, (B, 6, N))
+    feet = np.array([[0.2, -0.15, -0.3], [0.2, 0.15, -0.3], [-0.2, -0.15, -0.3], [-0.2, 0.15, -0.3]]).ravel()
+    U = np.empty((B, 24, N - 1))
+    U[:, 0:12] = np.tile(X[:, 0:3, :-1], (1, 4, 1)) + feet[None, :, None] + rng.uniform(-0.05, 0.05, (B, 12, N - 1))
+    U[:, 12:24] = rng.uniform(-20, 20, (B, 12, N - 1))
+    U[:, 14::3] = rng.uniform(0, 100, (B, 4, N - 1))
+    return X, U
+
+
+def _stored_trajectories(idx):
+    d = np.load(FIX)
+    return np.array([d["X"][b] for b in idx]), np.array([np.vstack([d["c"][b], d["f"][b]]) for b in idx])
+
+
+def _par(s, T, dt, n_steps, w):
+    par = s.tvlqr_default()
+    par.T, par.dt, par.n_steps, par.mass = T, dt, n_steps, w["mass"]
+    par.Q[:], par.F[:], par.R[:], par.Ib[:] = (w[k].ravel().tolist() for k in ("Q", "F", "R", "Ib"))
+    return par
+
+
+def _check(P, K, X, U, T, dt, n_steps, w, which):
+    """P [n_steps, 24, 24] and K [n_steps, 12, 24] of the trajectories `which` against the restatement; worst errors."""
+    wp = wk = 0.0
+    for i in which:
+        Pr, Kr = tvlqr_ref.riccati_backward(X[i], U[i], T, w["Q"], w["R"], w["F"], dt, n_steps, w["Ib"], w["mass"])
+        if P is not None:
+            e = np.max(np.abs(P[i] - Pr)) / max(1.0, np.abs(Pr).max())
+            assert e <= 1e-10, (i, e)
+            wp = max(wp, e)
+        if K is not None:
+            e = np.max(np.abs(K[i] - Kr)) / max(1.0, np.abs(Kr).max())
+            assert e <= 1e-10, (i, e)
+            wk = max(wk, e)
+    return wp, wk
+
+
+def _xs(X, U):
+    return np.array([np.concatenate([x.T.ravel(), u.T.ravel()]) for x, u in zip(X, U)])
+
+
+# (N, T, dt, n_steps, trajectories): every time point on a knot (dt = T/(N-1) and 2T/(N-1)), the reference's step on
+# another horizon, one time point only, a long pass of 301 steps
+TVLQR_CASES = [(21, 0.5, 0.5 / 20, 21, "random"), (30, 0.3, 2 * 0.3 / 29, 15, "random"), (41, 0.45, 0.022, 21, "random"),
+               (41, 0.6, 0.022, 1, "stored"), (41, 0.6, 0.002, 301, "stored")]
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("N,T,dt,n_steps,traj", TVLQR_CASES)
+def test_gpu_tvlqr_full_weights_and_other_grids(N, T, dt, n_steps, traj):
+    rng = np.random.default_rng(N * 1000 + n_steps)
+    w = _weights(rng)
+    X, U = _random_trajectories(rng, N, 4) if traj == "random" else _stored_trajectories([0, 2, 17])
+    s = lc.LandingSolver(N=N)
+    P, K = s.tvlqr(_xs(X, U), _par(s, T, dt, n_steps, w))
+    s.close()
+    wp, wk = _check(P, K, X, U, T, dt, n_steps, w, range(len(X)))
+    print("tvlqr N=%d T=%g dt=%g n_steps=%d: worst rel. error P %.2e, K %.2e" % (N, T, dt, n_steps, wp, wk))
+
+
+@pytest.mark.gpu
+def test_gpu_tvlqr_single_outputs_device_buffers_and_a_large_batch():
+    """P_out or K_out NULL (each alone) through the C ABI, device buffers, and B = 300 CTAs checked on a sample."""
+    import ctypes
+    import torch
+    N, B, T, dt, n_steps = 21, 300, 0.6, 0.022, 28
+    rng = np.random.default_rng(300)
+    w = _weights(rng)
+    X, U = _random_trajectories(rng, N, B)
+    xs = _xs(X, U)
+    s = lc.LandingSolver(N=N)
+    par = _par(s, T, dt, n_steps, w)
+    P, K = s.tvlqr(xs, par)
+    wp, wk = _check(P, K, X, U, T, dt, n_steps, w, [0, 1, 127, 128, 255, 299])
+    print("tvlqr B=%d: worst rel. error P %.2e, K %.2e" % (B, wp, wk))
+    dp = ctypes.POINTER(ctypes.c_double)
+    Ponly, Konly = np.zeros_like(P[:3]), np.zeros_like(K[:3])
+    x3 = np.ascontiguousarray(xs[:3])
+    for Pp, Kp in ((Ponly, None), (None, Konly)):
+        rc = s.lib.landing_tvlqr_batch(s.ctx, 3, lc.HOST, ctypes.byref(par), x3.ctypes.data_as(dp),
+                                       None if Pp is None else Pp.ctypes.data_as(dp),
+                                       None if Kp is None else Kp.ctypes.data_as(dp))
+        assert rc == 0, s.lib.landing_last_error()
+    assert np.array_equal(Ponly, P[:3]) and np.array_equal(Konly, K[:3])
+    dev = torch.device("cuda:0")
+    xt = torch.tensor(xs[:5], device=dev)
+    Pt = torch.full((5, n_steps, 24, 24), float("nan"), dtype=torch.float64, device=dev)
+    Kt = torch.full((5, n_steps, 12, 24), float("nan"), dtype=torch.float64, device=dev)
+    rc = s.lib.landing_tvlqr_batch(s.ctx, 5, lc.DEVICE, ctypes.byref(par), ctypes.cast(xt.data_ptr(), dp),
+                                   ctypes.cast(Pt.data_ptr(), dp), ctypes.cast(Kt.data_ptr(), dp))
+    assert rc == 0, s.lib.landing_last_error()
+    s.synchronize()
+    assert np.array_equal(Pt.cpu().numpy(), P[:5]) and np.array_equal(Kt.cpu().numpy(), K[:5])
+    s.close()
