@@ -216,8 +216,8 @@ int landing_tvlqr_batch(landing_ctx *ctx, long long B, int memspace, const landi
  * generate_solver/generate_landingCtrller_KNITRO.m:34-193): +12 joint angles per knot, foot positions tied to the forward
  * kinematics of the legs (get_forward_kin_foot.m:4-25), joint-torque limits tau = J_f' (-R' f) (get_foot_jacobians_mc.m:12-24),
  * joint limits, XYZ rotation convention (rpyToRotMat_xyz.m:2).  Batched constraint values and sparse Jacobian (CCS value
- * array, pattern from landing_kino_sparsity) -- the functions an NLP solver iterates on; the interior-point kernel itself
- * solves the SRB formulations only.  x[B x n_x] = [X(:); jpos(:); U(:)] per scenario (Opti variable order :45-51),
+ * array, pattern from landing_kino_sparsity) and, below, the Lagrangian Hessian (landing_kino_hess_batch) -- the
+ * functions an NLP solver iterates on; the interior-point kernel itself solves the SRB formulations only.  x[B x n_x] = [X(:); jpos(:); U(:)] per scenario (Opti variable order :45-51),
  * g[B x m], jac[B x nnz]; dims = {N, n_x = 12N + 36(N-1), m = 48 + 141(N-2) + 117, nnz}.  The row map and the bounds
  * lbg / ubg are restated in oracle/kino_ref.py (pinned to the stored solution generate_solver/prevSoln.mat). */
 typedef struct landing_kino_problem {
@@ -252,6 +252,17 @@ int landing_kino_setup_batch(landing_ctx *ctx, long long B, int memspace, int la
                              const double *drops, const double *x_srb, double *lbg, double *ubg, double *x0);
 int landing_kino_cost_batch(landing_ctx *ctx, long long B, int memspace, int layout, const landing_kino_setup *ks,
                             const double *x, double *f, double *grad_f);
+
+/* Lagrangian Hessian of the kino-dynamic NLP: H = d2/dx2 (lam_f f(x) + lam_g' g(x)), f the terminal cost of
+ * landing_kino_cost_batch, g the constraint function of landing_kino_eval_batch (the signs of CasADi's nlp_hess_l), as
+ * the CCS value array of its UPPER triangle (row <= col; the convention of landing_sparsity(ctx, 1)).  Exact
+ * second derivatives of the same knot function.  Every entry of hess is written on every call. */
+/* upper-triangle CCS {nrow, ncol, colind[ncol+1], row[nnz]} of the Lagrangian Hessian; host, library-owned, no GPU */
+const long long *landing_kino_hess_sparsity(int n_knots);
+/* hess[B x nnzH]; x [B x n_x]; lam_f [B] and lam_g [B x m]: NULL = all zero; ks (QN, q/qd_term_ref) required when lam_f != NULL */
+int landing_kino_hess_batch(landing_ctx *ctx, long long B, int memspace, int layout, const landing_kino_problem *pb,
+                            const landing_kino_setup *ks, const double *x, const double *lam_f,
+                            const double *lam_g, double *hess);
 
 /* Measured FP64 FMA throughput of the context's device in TFLOP/s (a DFMA micro-kernel timed with CUDA
  * events): the roofline denominator of the interior-point kernel, which is FP64-pipe bound by design. */

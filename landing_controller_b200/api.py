@@ -116,6 +116,12 @@ def load_library(path=LIB_PATH):
                                                  ctypes.POINTER(KinoSetup), _dp, _dp, _dp, _dp, _dp]
         lib.landing_kino_cost_batch.argtypes = [ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int, ctypes.c_int,
                                                 ctypes.POINTER(KinoSetup), _dp, _dp, _dp]
+    if hasattr(lib, "landing_kino_hess_batch"):
+        lib.landing_kino_hess_sparsity.restype = ctypes.POINTER(ctypes.c_longlong)
+        lib.landing_kino_hess_sparsity.argtypes = [ctypes.c_int]
+        lib.landing_kino_hess_batch.argtypes = [ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int, ctypes.c_int,
+                                                ctypes.POINTER(KinoProblem), ctypes.POINTER(KinoSetup), _dp, _dp, _dp,
+                                                _dp]
     lib.landing_launch_count.restype = ctypes.c_longlong
     lib.landing_launch_count.argtypes = [ctypes.c_void_p]
     if hasattr(lib, "landing_fp64_peak"):
@@ -439,6 +445,42 @@ class LandingSolver:
         self._check(self.lib.landing_kino_cost_batch(self.ctx, B, HOST, AOS, ctypes.byref(ks), _ptr(x), _ptr(f), _ptr(gf)),
                     "landing_kino_cost_batch")
         return f, gf
+
+    def kino_hess_sparsity(self):
+        """Upper-triangle CCS pattern of the Lagrangian Hessian of the kino-dynamic NLP: (colind [nx + 1], row [nnz])."""
+        sp = self.lib.landing_kino_hess_sparsity(self.N)
+        if not sp:
+            raise RuntimeError("landing_kino_hess_sparsity: %s" % self.lib.landing_last_error().decode())
+        nx = sp[1]
+        a = np.ctypeslib.as_array(sp, shape=(2 + nx + 1 + sp[2 + nx],))
+        return a[2:2 + nx + 1].copy(), a[2 + nx + 1:].copy()
+
+    def kino_hess_host(self, x, pb, lam_f=None, lam_g=None, ks=None, layout=AOS):
+        """CCS value array [B, nnzH] of the upper triangle of d2/dx2 (lam_f f + lam_g' g) of the kino-dynamic NLP
+        (host arrays; layout SOA: [n, B]).  lam_f [B], lam_g [B, m]: None = zero; ks: QN of the terminal cost (default
+        landing_kino_setup when lam_f is given)."""
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        B = x.shape[0] if layout == AOS else x.shape[1]
+        nnz = len(self.kino_hess_sparsity()[1])
+        if lam_f is not None:
+            lam_f = np.ascontiguousarray(lam_f, dtype=np.float64)
+            ks = ks or self.kino_setup_data()
+        if lam_g is not None:
+            lam_g = np.ascontiguousarray(lam_g, dtype=np.float64)
+        hess = np.zeros((B, nnz) if layout == AOS else (nnz, B))
+        self._check(self.lib.landing_kino_hess_batch(self.ctx, B, HOST, layout, ctypes.byref(pb),
+                                                     None if ks is None else ctypes.byref(ks), _ptr(x), _ptr(lam_f),
+                                                     _ptr(lam_g), _ptr(hess)), "landing_kino_hess_batch")
+        return hess
+
+    def kino_hess_device(self, x, pb, hess, lam_f=None, lam_g=None, ks=None, layout=SOA):
+        """Same with CUDA torch tensors already in HBM (enqueued on the library stream)."""
+        B = x.shape[0] if layout == AOS else x.shape[1]
+        if lam_f is not None:
+            ks = ks or self.kino_setup_data()
+        self._check(self.lib.landing_kino_hess_batch(self.ctx, B, DEVICE, layout, ctypes.byref(pb),
+                                                     None if ks is None else ctypes.byref(ks), _ptr(x), _ptr(lam_f),
+                                                     _ptr(lam_g), _ptr(hess)), "landing_kino_hess_batch")
 
     def synchronize(self):
         self._check(self.lib.landing_synchronize(self.ctx), "landing_synchronize")

@@ -59,6 +59,9 @@ struct landing_ctx {
   // kino-dynamic NLP (landing_kino_eval_batch): host plan and its device tables, made on first use
   std::shared_ptr<const KinoPlan> kino;
   int* d_kino = nullptr;
+  // its Lagrangian Hessian (landing_kino_hess_batch): pattern, writer and row-mask tables, made on first use
+  std::shared_ptr<const KinoHessPlan> khess;
+  int* d_khess = nullptr;
 };
 
 // dt[0..N-2] of this call on the device (stream-ordered): the caller's vector or the uniform T/(N-1)
@@ -253,6 +256,7 @@ void landing_destroy(landing_ctx* c) {
   solver_free(c->ws);
   if (c->d_maps) cudaFree(c->d_maps);
   if (c->d_kino) cudaFree(c->d_kino);
+  if (c->d_khess) cudaFree(c->d_khess);
   delete c;  // (the grow-only buffers)
   if (st) cudaStreamDestroy(st);
 }
@@ -397,6 +401,74 @@ int landing_kino_eval_batch(landing_ctx* c, long long B, int memspace, int layou
   soa_to_aos(c, B, pc, 3);
   CU(cudaGetLastError());
   return stage_out(c, memspace, pc, 3);
+}
+
+static std::shared_ptr<const KinoHessPlan> get_kino_hess_plan(int N) {
+  static std::mutex mu;
+  static std::map<int, std::shared_ptr<const KinoHessPlan>> cache;
+  std::lock_guard<std::mutex> lk(mu);
+  auto it = cache.find(N);
+  if (it != cache.end()) return it->second;
+  auto pl = std::make_shared<const KinoHessPlan>(make_kino_hess_plan(N));
+  cache[N] = pl;
+  return pl;
+}
+
+const long long* landing_kino_hess_sparsity(int N) {
+  if (N < 3) return nullptr;
+  auto pl = get_kino_hess_plan(N);
+  if (!pl->err.empty()) {
+    g_err = pl->err;
+    return nullptr;
+  }
+  return pl->sparsity.data();
+}
+
+int landing_kino_hess_batch(landing_ctx* c, long long B, int memspace, int layout, const landing_kino_problem* pb,
+                            const landing_kino_setup* ks, const double* x, const double* lam_f, const double* lam_g,
+                            double* hess) {
+  if (!c || !pb || !pb->dt || !x || !hess || B < 0 || (lam_f && !ks))
+    return fail(LANDING_ERR_ARG, "landing_kino_hess_batch: bad arguments (lam_f needs ks)");
+  if (B == 0) return LANDING_OK;
+  DeviceGuard guard_(c->device);
+  if (!c->khess) {
+    auto pl = get_kino_hess_plan(c->N);
+    if (!pl->err.empty()) return fail(LANDING_ERR_ARG, pl->err);
+    const size_t n = pl->hpos.size() + pl->cpos.size() + pl->rows.size();
+    CU(cudaMalloc(&c->d_khess, sizeof(int) * n));
+    CU(cudaMemcpy(c->d_khess, pl->hpos.data(), sizeof(int) * pl->hpos.size(), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(c->d_khess + pl->hpos.size(), pl->cpos.data(), sizeof(int) * 12, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(c->d_khess + pl->hpos.size() + 12, pl->rows.data(), sizeof(unsigned) * pl->rows.size(),
+                  cudaMemcpyHostToDevice));
+    c->khess = pl;
+  }
+  const KinoHessPlan& pl = *c->khess;
+  const long long m = 48 + 141LL * (c->N - 2) + 117;
+  int rc = stage_dt(c, pb->dt, 0.0);
+  if (rc) return rc;
+  // x, lam_g and hess of AoS batches on transposed copies (landing_kino_eval_batch); lam_f is [B] in both layouts
+  Piece pc[4] = {input(x, pl.nx * B), input(lam_g, m * B), output(hess, pl.nnz * B), input(lam_f, B)};
+  rc = stage_in(c, memspace, pc, 4);
+  if (!rc) rc = aos_to_soa(c, B, &layout, pc, 3);
+  if (rc) return rc;
+  KinoHessArgs a{};
+  a.N = c->N; a.B = B;
+  a.x = make_cview(pc[0].at<const double>(), pl.nx, B, layout);
+  a.lam_g = make_cview(pc[1].at<const double>(), m, B, layout);
+  a.hess = make_view(pc[2].at<double>(), pl.nnz, B, layout);
+  a.lam_f = make_cview(pc[3].at<const double>(), 1, B, layout);
+  a.pr.mu = pb->mu; a.pr.mass = pb->mass;
+  for (int i = 0; i < 3; i++) { a.pr.Ib[i] = pb->Ib[i]; a.pr.Ib_inv[i] = pb->Ib_inv[i]; }
+  for (int i = 0; i < 12; i++) a.QN[i] = lam_f ? ks->QN[i] : 0.0;
+  a.dtv = c->d_dt.as<double>();
+  a.hpos = c->d_khess;
+  a.cpos = c->d_khess + pl.hpos.size();
+  a.rows = reinterpret_cast<const unsigned*>(c->d_khess + pl.hpos.size() + 12);
+  c->launches += launch_kino_hess(a, c->stream);
+  CU(cudaGetLastError());
+  soa_to_aos(c, B, pc, 3);
+  CU(cudaGetLastError());
+  return stage_out(c, memspace, pc, 4);
 }
 
 int landing_fp64_peak(landing_ctx* c, double* tflops) {

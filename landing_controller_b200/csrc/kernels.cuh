@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <string>
 #include <vector>
 
 #include "../../include/landing_b200.h"
@@ -59,6 +60,13 @@ struct TvlqrArgs {
 int launch_tvlqr(const TvlqrArgs& a, long long B, cudaStream_t st);
 
 // kino-dynamic NLP (kino.cu): host plan (sizes, CCS pattern, scatter tables) and the batched evaluation
+__host__ __device__ inline long long kino_col(int N, int k, int v) {  // knot-local input v of knot k -> column of x
+  if (v < 12) return 12LL * k + v;
+  if (v < 24) return 12LL * N + 12LL * k + (v - 12);
+  if (v < 48) return 12LL * N + 12LL * (N - 1) + 24LL * k + (v - 24);
+  if (v < 60) return 12LL * (k + 1) + (v - 48);
+  return 12LL * N + 12LL * (N - 1) + 24LL * (k + 1) + (v - 60);
+}
 struct KinoPlan {
   int N = 0;
   long long nx = 0, m = 0, nnz = 0;
@@ -88,6 +96,29 @@ struct KinoSetupArgs {
 };
 int launch_kino_setup(const KinoSetupArgs& a, cudaStream_t st);
 int launch_kino_cost(const KinoSetupArgs& a, cudaStream_t st);
+// Lagrangian Hessian of the kino-dynamic NLP (kino_hess.cu): upper-triangle CCS pattern and the writer of every entry
+struct KinoHessPlan {
+  int N = 0;
+  long long nx = 0, nnz = 0;
+  std::vector<long long> sparsity;  // CasADi CCS {nx, nx, colind[nx+1], row[nnz]}, upper triangle
+  std::vector<int> hpos;            // [knot][pass][3 x 3] -> CCS position or -1
+  std::vector<unsigned> rows;       // [knot class][pass][5 words]: rows with a second-order part in the pass's block
+  std::vector<int> cpos;            // [12] terminal-cost diagonal of X_{N-1}
+  std::string err;                  // non-empty: the pair table misses a non-zero block, or an entry has two writers
+};
+KinoHessPlan make_kino_hess_plan(int N);
+struct KinoHessArgs {
+  int N;
+  long long B;
+  CView x, lam_f, lam_g;
+  View hess;
+  kino::Params pr;
+  double QN[12];      // 0 without lam_f
+  const double* dtv;  // knot spacings (device)
+  const int *hpos, *cpos;
+  const unsigned* rows;
+};
+int launch_kino_hess(const KinoHessArgs& a, cudaStream_t st);
 
 // returns number of kernel launches issued
 int launch_eval(const EvalArgs& a, cudaStream_t st);

@@ -24,14 +24,6 @@ using kino::NIN;
 using kino::ROWS_INT;
 using kino::ROWS_LAST;
 
-__host__ __device__ inline long long kino_col(int N, int k, int v) {  // knot-local input v of knot k -> column of x
-  if (v < 12) return 12LL * k + v;
-  if (v < 24) return 12LL * N + 12LL * k + (v - 12);
-  if (v < 48) return 12LL * N + 12LL * (N - 1) + 24LL * k + (v - 24);
-  if (v < 60) return 12LL * (k + 1) + (v - 48);
-  return 12LL * N + 12LL * (N - 1) + 24LL * (k + 1) + (v - 60);
-}
-
 struct GSink {
   View g;
   long long b, base;

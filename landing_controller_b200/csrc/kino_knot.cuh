@@ -2,14 +2,15 @@
 // (SURVEY 8 f-2): generate_solver/generate_landingCtrller_KNITRO.m:107-193 with get_forward_kin_foot.m:4-25 on the
 // 18-body model of get_robot_model.m:134-244 (closed form of that chain), get_foot_jacobians_mc.m:3-24,
 // rpyToRotMat_xyz.m:2, Binv.m:13-17.  Templated on the scalar type of every input block: double for the constraint values, DualN
-// (value + tangents) on the seeded block for the Jacobian columns -- exact derivatives, no hand-derived entries.  Host
-// and device.
+// (value + tangents) on the seeded block for the Jacobian columns, Dual2 (second order) on two seeded triples for the
+// blocks of the Lagrangian Hessian -- exact derivatives, no hand-derived entries.  Host and device.
 //
 // Knot-local inputs (72): X_k 0..11 (r, rpy, omega_body, v_world) | jpos_k 12..23 | U_k 24..47 (c[4x3], f[4x3]) |
 // X_{k+1} 48..59 | c_{k+1} 60..71 (unused by the last knot).  Knot-local rows (141; 117 for the last knot, whose 24
 // no-slip rows are absent): see the row map in oracle/kino_ref.py.
 #pragma once
 #include <cmath>
+#include <type_traits>
 
 namespace srb {
 namespace kino {
@@ -102,9 +103,122 @@ template <int K> KHD void sincos_s(const DualN<K>& a, DualN<K>& s, DualN<K>& c) 
 }
 KHD void sincos_s(double a, double& s, double& c) { s = sin(a); c = cos(a); }
 using Dual1 = DualN<1>;  // one tangent (host-side pattern probing)
+
+// Second order, forward over forward: value, three tangents in seed set A, three in seed set B and the 3 x 3 block of
+// mixed second derivatives h[i][j] = d2 / dA_i dB_j.  A Hessian pass types the block(s) of two input triples this way
+// (seeds A on one triple, B on the other; both on the same triple for a diagonal block) and every other block a plain
+// double, so the knot function above runs unchanged and whatever does not depend on either triple stays ordinary double
+// arithmetic.
+struct Dual2 {
+  double v, a[3], b[3], h[3][3];
+  KHD Dual2() : Dual2(0.0) {}
+  KHD Dual2(double x) : v(x) {
+#pragma unroll
+    for (int i = 0; i < 3; i++) {
+      a[i] = 0.0; b[i] = 0.0;
+#pragma unroll
+      for (int j = 0; j < 3; j++) h[i][j] = 0.0;
+    }
+  }
+};
+KHD Dual2 operator+(const Dual2& x, const Dual2& y) {
+  Dual2 r; r.v = x.v + y.v;
+#pragma unroll
+  for (int i = 0; i < 3; i++) {
+    r.a[i] = x.a[i] + y.a[i]; r.b[i] = x.b[i] + y.b[i];
+#pragma unroll
+    for (int j = 0; j < 3; j++) r.h[i][j] = x.h[i][j] + y.h[i][j];
+  }
+  return r;
+}
+KHD Dual2 operator-(const Dual2& x) {
+  Dual2 r; r.v = -x.v;
+#pragma unroll
+  for (int i = 0; i < 3; i++) {
+    r.a[i] = -x.a[i]; r.b[i] = -x.b[i];
+#pragma unroll
+    for (int j = 0; j < 3; j++) r.h[i][j] = -x.h[i][j];
+  }
+  return r;
+}
+KHD Dual2 operator-(const Dual2& x, const Dual2& y) {
+  Dual2 r; r.v = x.v - y.v;
+#pragma unroll
+  for (int i = 0; i < 3; i++) {
+    r.a[i] = x.a[i] - y.a[i]; r.b[i] = x.b[i] - y.b[i];
+#pragma unroll
+    for (int j = 0; j < 3; j++) r.h[i][j] = x.h[i][j] - y.h[i][j];
+  }
+  return r;
+}
+KHD Dual2 operator*(const Dual2& x, const Dual2& y) {
+  Dual2 r; r.v = x.v * y.v;
+#pragma unroll
+  for (int i = 0; i < 3; i++) {
+    r.a[i] = x.a[i] * y.v + x.v * y.a[i];
+    r.b[i] = x.b[i] * y.v + x.v * y.b[i];
+  }
+#pragma unroll
+  for (int i = 0; i < 3; i++)
+#pragma unroll
+    for (int j = 0; j < 3; j++)
+      r.h[i][j] = x.h[i][j] * y.v + x.v * y.h[i][j] + x.a[i] * y.b[j] + y.a[i] * x.b[j];
+  return r;
+}
+KHD Dual2 operator/(const Dual2& x, const Dual2& y) {  // q = x / y from x = q y
+  Dual2 r; const double iy = 1.0 / y.v; r.v = x.v * iy;
+#pragma unroll
+  for (int i = 0; i < 3; i++) {
+    r.a[i] = (x.a[i] - r.v * y.a[i]) * iy;
+    r.b[i] = (x.b[i] - r.v * y.b[i]) * iy;
+  }
+#pragma unroll
+  for (int i = 0; i < 3; i++)
+#pragma unroll
+    for (int j = 0; j < 3; j++)
+      r.h[i][j] = (x.h[i][j] - r.v * y.h[i][j] - r.a[i] * y.b[j] - y.a[i] * r.b[j]) * iy;
+  return r;
+}
+// mixed with plain doubles
+KHD Dual2 operator*(const Dual2& x, double y) {
+  Dual2 r; r.v = x.v * y;
+#pragma unroll
+  for (int i = 0; i < 3; i++) {
+    r.a[i] = x.a[i] * y; r.b[i] = x.b[i] * y;
+#pragma unroll
+    for (int j = 0; j < 3; j++) r.h[i][j] = x.h[i][j] * y;
+  }
+  return r;
+}
+KHD Dual2 operator*(double x, const Dual2& y) { return y * x; }
+KHD Dual2 operator+(const Dual2& x, double y) { Dual2 r = x; r.v = x.v + y; return r; }
+KHD Dual2 operator+(double x, const Dual2& y) { Dual2 r = y; r.v = x + y.v; return r; }
+KHD Dual2 operator-(const Dual2& x, double y) { Dual2 r = x; r.v = x.v - y; return r; }
+KHD Dual2 operator-(double x, const Dual2& y) { Dual2 r = -y; r.v = x - y.v; return r; }
+KHD Dual2 operator/(const Dual2& x, double y) { return x * (1.0 / y); }
+KHD Dual2 operator/(double x, const Dual2& y) { return Dual2(x) / y; }
+KHD void sincos_s(const Dual2& x, Dual2& s, Dual2& c) {
+  const double sv = sin(x.v), cv = cos(x.v);
+  s.v = sv; c.v = cv;
+#pragma unroll
+  for (int i = 0; i < 3; i++) {
+    s.a[i] = cv * x.a[i]; s.b[i] = cv * x.b[i];
+    c.a[i] = -sv * x.a[i]; c.b[i] = -sv * x.b[i];
+  }
+#pragma unroll
+  for (int i = 0; i < 3; i++)
+#pragma unroll
+    for (int j = 0; j < 3; j++) {
+      const double ab = x.a[i] * x.b[j];
+      s.h[i][j] = cv * x.h[i][j] - sv * ab;
+      c.h[i][j] = -sv * x.h[i][j] - cv * ab;
+    }
+}
+
 // result type of an arithmetic expression of two scalar types
 template <class A, class B> struct Promote { using type = A; };
 template <int K> struct Promote<double, DualN<K>> { using type = DualN<K>; };
+template <> struct Promote<double, Dual2> { using type = Dual2; };
 template <class A, class B> using Pr = typename Promote<A, B>::type;
 
 struct Params {
@@ -322,6 +436,76 @@ KHD void jac_pass(const double* x, double h, const Params& pr, Sink& s) {
     if constexpr (blk == 7) knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, x + 12, x + 24, x + 36, t, x + 60, h, pr, s, mask);
     if constexpr (blk == 8) knot_rows_h<LAST>(x, x + 3, x + 6, x + 9, x + 12, x + 24, x + 36, x + 48, t, h, pr, s, mask);
   }
+}
+
+// Hessian passes.  Triples of knot-local inputs: 0 r | 1 rpy | 2 omega | 3 v | 4 + l joint angles, 8 + l foot position,
+// 12 + l force of leg l | 16..19 next state | 20 + l next foot position.  A pass is an ordered pair of triples (a <= b)
+// whose cross block d2 L / dz_a dz_b is non-zero somewhere: it runs the knot function with the block(s) of the two
+// triples typed Dual2 (seeds A on a, B on b), restricted to the row groups both triples reach, and owns the 3 x 3 block
+// (its upper triangle when a == b).  The table is grouped by weight (the kernels of kino_hess.cu): the pairs with rpy,
+// whose rotation matrix makes every row second order; the joint-angle pairs; the rest.  The host plan derives the
+// non-zero pairs by probing every one of the 300 triple pairs and refuses a table that misses one.
+constexpr int HESS_PASSES = 45, HESS_RPY_END = 15, HESS_JPOS_END = 23;
+KHD constexpr int hess_pair(int P) {  // pass -> 32 a + b
+  constexpr int t[HESS_PASSES] = {
+      // [0, 15): with rpy -- r, rpy, omega, and the joint angles, foot position and force of each leg
+      0 * 32 + 1, 1 * 32 + 1, 1 * 32 + 2, 1 * 32 + 4, 1 * 32 + 5, 1 * 32 + 6, 1 * 32 + 7, 1 * 32 + 8, 1 * 32 + 9,
+      1 * 32 + 10, 1 * 32 + 11, 1 * 32 + 12, 1 * 32 + 13, 1 * 32 + 14, 1 * 32 + 15,
+      // [15, 23): joint angles x joint angles, joint angles x force, by leg
+      4 * 32 + 4, 4 * 32 + 12, 5 * 32 + 5, 5 * 32 + 13, 6 * 32 + 6, 6 * 32 + 14, 7 * 32 + 7, 7 * 32 + 15,
+      // [23, 45): r x r, r x foot position, r x force, omega x omega, and per leg foot position x foot position,
+      // foot position x force, force x next foot position
+      0 * 32 + 0, 0 * 32 + 8, 0 * 32 + 9, 0 * 32 + 10, 0 * 32 + 11, 0 * 32 + 12, 0 * 32 + 13, 0 * 32 + 14, 0 * 32 + 15,
+      2 * 32 + 2, 8 * 32 + 8, 8 * 32 + 12, 9 * 32 + 9, 9 * 32 + 13, 10 * 32 + 10, 10 * 32 + 14, 11 * 32 + 11,
+      11 * 32 + 15, 12 * 32 + 20, 13 * 32 + 21, 14 * 32 + 22, 15 * 32 + 23};
+  return t[P];
+}
+KHD constexpr int tri_block(int t) { return t < 4 ? t : t < 8 ? 4 : t < 12 ? 5 : t < 16 ? 6 : t < 20 ? 7 : 8; }
+KHD constexpr int block_base(int blk) { return blk < 4 ? 3 * blk : 12 * (blk - 3); }
+template <int P> struct HessPassOf {  // pass -> (triples a <= b, row groups both reach)
+  static constexpr int a = hess_pair(P) / 32, b = hess_pair(P) % 32;
+  static constexpr unsigned mask = reach(3 * a) & reach(3 * b);
+};
+KHD constexpr bool hess_pass_in_knot(bool last, int P) { return !(last && hess_pair(P) % 32 >= 20); }  // (no c_{k+1})
+
+// One input block of a Hessian pass: the caller's doubles, or -- if the block holds triple a or b -- a Dual2 copy seeded
+// with tangent A_i on element i of triple a and B_j on element j of triple b.
+template <int BLK, int TA, int TB> struct HessBlock {
+  static constexpr bool typed = tri_block(TA) == BLK || tri_block(TB) == BLK;
+  static constexpr int base = block_base(BLK), len = BLK < 4 ? 3 : 12;
+  using T = typename std::conditional<typed, Dual2, double>::type;
+  T buf[typed ? len : 1];
+  const T* p;
+  KHD explicit HessBlock(const double* x) {
+    if constexpr (typed) {
+#pragma unroll
+      for (int i = 0; i < len; i++) {
+        buf[i] = Dual2(x[base + i]);
+        if ((base + i) / 3 == TA) buf[i].a[(base + i) % 3] = 1.0;
+        if ((base + i) / 3 == TB) buf[i].b[(base + i) % 3] = 1.0;
+      }
+      p = buf;
+    } else {
+      p = x + base;
+    }
+  }
+};
+
+// Pass P on the knot-local inputs x: out(rho, Dual2) gets d2 row / dz_{3a+i} dz_{3b+j} as h[i][j] (out(rho, double): a
+// row that depends on neither triple).
+template <bool LAST, int P, class Sink>
+KHD void hess_pass(const double* x, double h, const Params& pr, Sink& s) {
+  constexpr int A = HessPassOf<P>::a, B = HessPassOf<P>::b;
+  const HessBlock<0, A, B> b0(x);
+  const HessBlock<1, A, B> b1(x);
+  const HessBlock<2, A, B> b2(x);
+  const HessBlock<3, A, B> b3(x);
+  const HessBlock<4, A, B> b4(x);
+  const HessBlock<5, A, B> b5(x);
+  const HessBlock<6, A, B> b6(x);
+  const HessBlock<7, A, B> b7(x);
+  const HessBlock<8, A, B> b8(x);
+  knot_rows_h<LAST>(b0.p, b1.p, b2.p, b3.p, b4.p, b5.p, b6.p, b7.p, b8.p, h, pr, s, HessPassOf<P>::mask);
 }
 
 // Which thread of a (scenario, knot) quadruple owns row rho when the knot is split by leg (k_kino_g): the rows of leg l
