@@ -216,8 +216,8 @@ int landing_tvlqr_batch(landing_ctx *ctx, long long B, int memspace, const landi
  * generate_solver/generate_landingCtrller_KNITRO.m:34-193): +12 joint angles per knot, foot positions tied to the forward
  * kinematics of the legs (get_forward_kin_foot.m:4-25), joint-torque limits tau = J_f' (-R' f) (get_foot_jacobians_mc.m:12-24),
  * joint limits, XYZ rotation convention (rpyToRotMat_xyz.m:2).  Batched constraint values and sparse Jacobian (CCS value
- * array, pattern from landing_kino_sparsity) and, below, the Lagrangian Hessian (landing_kino_hess_batch) -- the
- * functions an NLP solver iterates on; the interior-point kernel itself solves the SRB formulations only.  x[B x n_x] = [X(:); jpos(:); U(:)] per scenario (Opti variable order :45-51),
+ * array, pattern from landing_kino_sparsity) and, below, the Lagrangian Hessian (landing_kino_hess_batch), gradient and
+ * KKT residuals (landing_kino_kkt_batch) -- the functions an NLP solver iterates on; the interior-point kernel itself solves the SRB formulations only.  x[B x n_x] = [X(:); jpos(:); U(:)] per scenario (Opti variable order :45-51),
  * g[B x m], jac[B x nnz]; dims = {N, n_x = 12N + 36(N-1), m = 48 + 141(N-2) + 117, nnz}.  The row map and the bounds
  * lbg / ubg are restated in oracle/kino_ref.py (pinned to the stored solution generate_solver/prevSoln.mat). */
 typedef struct landing_kino_problem {
@@ -263,6 +263,35 @@ const long long *landing_kino_hess_sparsity(int n_knots);
 int landing_kino_hess_batch(landing_ctx *ctx, long long B, int memspace, int layout, const landing_kino_problem *pb,
                             const landing_kino_setup *ks, const double *x, const double *lam_f,
                             const double *lam_g, double *hess);
+
+/* Lagrangian gradient and KKT residuals of the kino-dynamic NLP at a primal-dual point (x, lam_f, lam_g), with CasADi's
+ * sign convention L = lam_f f + lam_g' g (f the terminal cost of landing_kino_cost_batch, g the rows of
+ * landing_kino_eval_batch), per scenario:
+ *   grad_x    = lam_f grad f + J' lam_g                                     (CasADi nlp_grad: grad_gamma_x)
+ *   viol      = max_i max(lbg_i - g_i, g_i - ubg_i, 0); an infinite bound never counts
+ *   dual_inf  = max_j |grad_x_j|, unscaled.  The NLP has no variable bounds, so lam_x = -grad_x
+ *   compl_inf = max_i c_i over the inequality rows (lbg_i < ubg_i; equality rows are excluded),
+ *               c_i = max(lam_g_i, 0) |ubg_i - g_i| + max(-lam_g_i, 0) |g_i - lbg_i|; a multiplier of the wrong sign
+ *               for an infinite bound gives +inf (lam_g_i = 0 gives 0)
+ * A NaN in any input of a scenario (x, lam_f, lam_g, lbg, ubg), or in the g or grad_x computed from them, makes each of
+ * that scenario's viol / dual_inf / compl_inf NaN, and no other scenario's.  Results are deterministic: the same bits from
+ * run to run, in both layouts and both memory spaces.  grad_x is computed without forming J, and every entry is written
+ * on every call.  Every output may be NULL; B = 0 launches nothing. */
+typedef struct landing_kino_kkt_io {
+  const double *x;         /* [B x n_x], required */
+  const double *lam_f;     /* [B] in both layouts, NULL = 0 (needs ks) */
+  const double *lam_g;     /* [B x m], NULL = 0 */
+  const double *lbg, *ubg; /* [B x m], both or neither (landing_kino_setup_batch gives them) */
+  double *grad_x;          /* [B x n_x] */
+  double *viol;            /* [B]: needs lbg / ubg */
+  double *dual_inf;        /* [B] */
+  double *compl_inf;       /* [B]: needs lbg / ubg */
+} landing_kino_kkt_io;
+/* ks (QN, q/qd_term_ref of the cost) is required only when lam_f != NULL.  LANDING_ERR_ARG, with the context left
+ * usable: a NULL ctx / pb / pb->dt / io / x, B < 0, lam_f without ks, only one of lbg / ubg, viol or compl_inf without
+ * the bounds. */
+int landing_kino_kkt_batch(landing_ctx *ctx, long long B, int memspace, int layout, const landing_kino_problem *pb,
+                           const landing_kino_setup *ks, const landing_kino_kkt_io *io);
 
 /* Measured FP64 FMA throughput of the context's device in TFLOP/s (a DFMA micro-kernel timed with CUDA
  * events): the roofline denominator of the interior-point kernel, which is FP64-pipe bound by design. */

@@ -78,6 +78,11 @@ class KinoSetup(ctypes.Structure):
                 ("jpos_guess", ctypes.c_double * 3)]
 
 
+class KinoKktIO(ctypes.Structure):
+    """landing_kino_kkt_io: a primal-dual point of the kino-dynamic NLP and its Lagrangian gradient / KKT residuals."""
+    _fields_ = [(n, _dp) for n in ("x", "lam_f", "lam_g", "lbg", "ubg", "grad_x", "viol", "dual_inf", "compl_inf")]
+
+
 class SolveIO(ctypes.Structure):
     _fields_ = [("drops", _dp), ("x0", _dp), ("x_star", _dp), ("f_star", _dp), ("lam_g", _dp),
                 ("viol", _dp), ("status", _ip), ("iters", _ip)]
@@ -122,6 +127,10 @@ def load_library(path=LIB_PATH):
         lib.landing_kino_hess_batch.argtypes = [ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int, ctypes.c_int,
                                                 ctypes.POINTER(KinoProblem), ctypes.POINTER(KinoSetup), _dp, _dp, _dp,
                                                 _dp]
+    if hasattr(lib, "landing_kino_kkt_batch"):
+        lib.landing_kino_kkt_batch.argtypes = [ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int, ctypes.c_int,
+                                               ctypes.POINTER(KinoProblem), ctypes.POINTER(KinoSetup),
+                                               ctypes.POINTER(KinoKktIO)]
     lib.landing_launch_count.restype = ctypes.c_longlong
     lib.landing_launch_count.argtypes = [ctypes.c_void_p]
     if hasattr(lib, "landing_fp64_peak"):
@@ -481,6 +490,43 @@ class LandingSolver:
         self._check(self.lib.landing_kino_hess_batch(self.ctx, B, DEVICE, layout, ctypes.byref(pb),
                                                      None if ks is None else ctypes.byref(ks), _ptr(x), _ptr(lam_f),
                                                      _ptr(lam_g), _ptr(hess)), "landing_kino_hess_batch")
+
+    def kino_kkt_host(self, x, pb, lam_f=None, lam_g=None, lbg=None, ubg=None, ks=None, want=None, layout=AOS):
+        """Lagrangian gradient and KKT residuals of the kino-dynamic NLP at (x, lam_f, lam_g) (include/landing_b200.h:
+        landing_kino_kkt_batch).  Host arrays; layout SOA: [n, B] (lam_f and the [B] outputs are [B] in both layouts).
+        lam_f [B], lam_g [B, m]: None = zero; lbg / ubg [B, m]: landing_kino_setup_batch's bounds; ks: the cost data
+        (default landing_kino_setup when lam_f is given).  want: the outputs to compute, any of "grad_x", "viol",
+        "dual_inf", "compl_inf" (default: all four with bounds, else grad_x and dual_inf).  Returns a dict of them;
+        lam_x = -grad_x (the NLP has no variable bounds)."""
+        d = self.kino_dims()
+        c = (lambda a: None if a is None else np.ascontiguousarray(a, dtype=np.float64))
+        x, lam_f, lam_g, lbg, ubg = c(x), c(lam_f), c(lam_g), c(lbg), c(ubg)
+        B = x.shape[0] if layout == AOS else x.shape[1]
+        if lam_f is not None:
+            ks = ks or self.kino_setup_data()
+        if want is None:
+            want = ("grad_x", "viol", "dual_inf", "compl_inf") if lbg is not None else ("grad_x", "dual_inf")
+        out = {k: np.zeros(B) for k in want if k != "grad_x"}
+        if "grad_x" in want:
+            out["grad_x"] = np.zeros((B, d["nx"]) if layout == AOS else (d["nx"], B))
+        io = KinoKktIO(_ptr(x), _ptr(lam_f), _ptr(lam_g), _ptr(lbg), _ptr(ubg), _ptr(out.get("grad_x")),
+                       _ptr(out.get("viol")), _ptr(out.get("dual_inf")), _ptr(out.get("compl_inf")))
+        self._check(self.lib.landing_kino_kkt_batch(self.ctx, B, HOST, layout, ctypes.byref(pb),
+                                                    None if ks is None else ctypes.byref(ks), ctypes.byref(io)),
+                    "landing_kino_kkt_batch")
+        return out
+
+    def kino_kkt_device(self, x, pb, lam_f=None, lam_g=None, lbg=None, ubg=None, grad_x=None, viol=None, dual_inf=None,
+                        compl_inf=None, ks=None, layout=SOA):
+        """Same with CUDA torch tensors already in HBM (enqueued on the library stream); any output may be None."""
+        B = x.shape[0] if layout == AOS else x.shape[1]
+        if lam_f is not None:
+            ks = ks or self.kino_setup_data()
+        io = KinoKktIO(_ptr(x), _ptr(lam_f), _ptr(lam_g), _ptr(lbg), _ptr(ubg), _ptr(grad_x), _ptr(viol), _ptr(dual_inf),
+                       _ptr(compl_inf))
+        self._check(self.lib.landing_kino_kkt_batch(self.ctx, B, DEVICE, layout, ctypes.byref(pb),
+                                                    None if ks is None else ctypes.byref(ks), ctypes.byref(io)),
+                    "landing_kino_kkt_batch")
 
     def synchronize(self):
         self._check(self.lib.landing_synchronize(self.ctx), "landing_synchronize")

@@ -62,6 +62,8 @@ struct landing_ctx {
   // its Lagrangian Hessian (landing_kino_hess_batch): pattern, writer and row-mask tables, made on first use
   std::shared_ptr<const KinoHessPlan> khess;
   int* d_khess = nullptr;
+  // scratch of its KKT residuals (landing_kino_kkt_batch): g, and grad_x when the caller does not ask for it
+  DeviceBuf kkt;
 };
 
 // dt[0..N-2] of this call on the device (stream-ordered): the caller's vector or the uniform T/(N-1)
@@ -469,6 +471,89 @@ int landing_kino_hess_batch(landing_ctx* c, long long B, int memspace, int layou
   soa_to_aos(c, B, pc, 3);
   CU(cudaGetLastError());
   return stage_out(c, memspace, pc, 4);
+}
+
+// Launches of one call (B > 0, at least one output):
+//   6 gradient kernels            if grad_x or dual_inf is wanted
+// + 1 g kernel (k_kino_g)         if viol or compl_inf is wanted
+// + 1 residual kernel             if viol, dual_inf or compl_inf is wanted
+// + for AoS batches of B >= 64: 1 transpose of x, 1 of lam_g if given, 2 of lbg / ubg if given, 1 of grad_x if wanted.
+// For example grad_x alone: 6 (SoA) or 8 (AoS, B >= 64, lam_g given); all four outputs with lam_g and the bounds: 8 (SoA)
+// or 13 (AoS, B >= 64).
+int landing_kino_kkt_batch(landing_ctx* c, long long B, int memspace, int layout, const landing_kino_problem* pb,
+                           const landing_kino_setup* ks, const landing_kino_kkt_io* io) {
+  if (!c || !pb || !pb->dt || !io || !io->x || B < 0)
+    return fail(LANDING_ERR_ARG, "landing_kino_kkt_batch: bad arguments");
+  if (io->lam_f && !ks) return fail(LANDING_ERR_ARG, "landing_kino_kkt_batch: lam_f needs ks");
+  if (!io->lbg != !io->ubg) return fail(LANDING_ERR_ARG, "landing_kino_kkt_batch: give both lbg and ubg, or neither");
+  if ((io->viol || io->compl_inf) && !io->lbg)
+    return fail(LANDING_ERR_ARG, "landing_kino_kkt_batch: viol and compl_inf need lbg / ubg");
+  const bool want_grad = io->grad_x || io->dual_inf, want_g = io->viol || io->compl_inf;
+  const bool want_res = want_g || io->dual_inf;
+  if (B == 0 || (!want_grad && !want_res)) return LANDING_OK;
+  DeviceGuard guard_(c->device);
+  auto pl = get_kino_plan(c->N);
+  const long long nx = pl->nx, m = pl->m;
+  int rc = stage_dt(c, pb->dt, 0.0);
+  if (rc) return rc;
+  // x, lam_g, the bounds and grad_x of AoS batches on transposed copies (landing_kino_eval_batch); the others are [B]
+  Piece pc[9] = {input(io->x, nx * B),     input(io->lam_g, m * B), input(io->lbg, m * B), input(io->ubg, m * B),
+                 output(io->grad_x, nx * B), input(io->lam_f, B),   output(io->viol, B),   output(io->dual_inf, B),
+                 output(io->compl_inf, B)};
+  rc = stage_in(c, memspace, pc, 9);
+  if (!rc) rc = aos_to_soa(c, B, &layout, pc, 5);
+  if (rc) return rc;
+  // scratch (SoA): g [m x B], and grad_x [n_x x B] when only its norm is wanted
+  const bool own_grad = io->dual_inf && !io->grad_x;
+  CU(c->kkt.reserve(sizeof(double) * ((want_g ? m : 0) + (own_grad ? nx : 0)) * B));
+  double* const g_s = want_g ? c->kkt.as<double>() : nullptr;
+  double* const gx_s = own_grad ? c->kkt.as<double>() + (want_g ? m * B : 0) : nullptr;
+  const CView x = make_cview(pc[0].at<const double>(), nx, B, layout);
+  const View grad = own_grad ? make_view(gx_s, nx, B, LANDING_SOA) : make_view(pc[4].at<double>(), nx, B, layout);
+  kino::Params pr{pb->mu, pb->mass, {pb->Ib[0], pb->Ib[1], pb->Ib[2]}, {pb->Ib_inv[0], pb->Ib_inv[1], pb->Ib_inv[2]}};
+  if (want_grad) {
+    KinoGradArgs a{};
+    a.N = c->N; a.B = B;
+    a.x = x;
+    a.lam_f = make_cview(pc[5].at<const double>(), 1, B, layout);
+    a.lam_g = make_cview(pc[1].at<const double>(), m, B, layout);
+    a.grad = grad;
+    a.pr = pr;
+    for (int i = 0; i < 12; i++) {
+      a.QN[i] = io->lam_f ? ks->QN[i] : 0.0;
+      a.ref[i] = !io->lam_f ? 0.0 : i < 6 ? ks->q_term_ref[i] : ks->qd_term_ref[i - 6];
+    }
+    a.dtv = c->d_dt.as<double>();
+    c->launches += launch_kino_grad(a, c->stream);
+  }
+  if (want_g) {
+    KinoArgs a{};
+    a.N = c->N; a.B = B;
+    a.x = x;
+    a.g = make_view(g_s, m, B, LANDING_SOA);
+    a.pr = pr;
+    a.dtv = c->d_dt.as<double>();
+    c->launches += launch_kino(a, true, false, c->stream);
+  }
+  if (want_res) {
+    KinoKktArgs a{};
+    a.B = B; a.m = m; a.nx = nx;
+    a.x = x;
+    a.lam_f = make_cview(pc[5].at<const double>(), 1, B, layout);
+    a.lam_g = make_cview(pc[1].at<const double>(), m, B, layout);
+    a.lbg = make_cview(pc[2].at<const double>(), m, B, layout);
+    a.ubg = make_cview(pc[3].at<const double>(), m, B, layout);
+    a.g = make_view(g_s, m, B, LANDING_SOA);
+    a.grad = io->dual_inf ? grad : View{nullptr, 0, 0};
+    a.viol = make_view(pc[6].at<double>(), 1, B, layout);
+    a.dual_inf = make_view(pc[7].at<double>(), 1, B, layout);
+    a.compl_inf = make_view(pc[8].at<double>(), 1, B, layout);
+    c->launches += launch_kino_kkt(a, c->stream);
+  }
+  CU(cudaGetLastError());
+  soa_to_aos(c, B, pc, 5);
+  CU(cudaGetLastError());
+  return stage_out(c, memspace, pc, 9);
 }
 
 int landing_fp64_peak(landing_ctx* c, double* tflops) {

@@ -60,13 +60,7 @@ struct TvlqrArgs {
 int launch_tvlqr(const TvlqrArgs& a, long long B, cudaStream_t st);
 
 // kino-dynamic NLP (kino.cu): host plan (sizes, CCS pattern, scatter tables) and the batched evaluation
-__host__ __device__ inline long long kino_col(int N, int k, int v) {  // knot-local input v of knot k -> column of x
-  if (v < 12) return 12LL * k + v;
-  if (v < 24) return 12LL * N + 12LL * k + (v - 12);
-  if (v < 48) return 12LL * N + 12LL * (N - 1) + 24LL * k + (v - 24);
-  if (v < 60) return 12LL * (k + 1) + (v - 48);
-  return 12LL * N + 12LL * (N - 1) + 24LL * (k + 1) + (v - 60);
-}
+__host__ __device__ inline long long kino_col(int N, int k, int v) { return kino::knot_col(N, k, v); }
 struct KinoPlan {
   int N = 0;
   long long nx = 0, m = 0, nnz = 0;
@@ -119,6 +113,24 @@ struct KinoHessArgs {
   const unsigned* rows;
 };
 int launch_kino_hess(const KinoHessArgs& a, cudaStream_t st);
+// Lagrangian gradient and KKT residuals of the kino-dynamic NLP (kino_grad.cu)
+struct KinoGradArgs {
+  int N;
+  long long B;
+  CView x, lam_f, lam_g;  // lam_f / lam_g NULL: no cost / no row terms
+  View grad;
+  kino::Params pr;
+  double QN[12], ref[12];  // terminal cost (with lam_f)
+  const double* dtv;       // knot spacings (device)
+};
+int launch_kino_grad(const KinoGradArgs& a, cudaStream_t st);
+struct KinoKktArgs {
+  long long B, m, nx;
+  CView x, lam_f, lam_g, lbg, ubg;  // any may be NULL but x
+  View g, grad;                     // g(x) when viol / compl_inf are wanted, grad_x when dual_inf is; else NULL
+  View viol, dual_inf, compl_inf;   // [1 x B], any may be NULL
+};
+int launch_kino_kkt(const KinoKktArgs& a, cudaStream_t st);
 
 // returns number of kernel launches issued
 int launch_eval(const EvalArgs& a, cudaStream_t st);

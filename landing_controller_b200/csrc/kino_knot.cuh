@@ -225,6 +225,15 @@ struct Params {
   double mu, mass, Ib[3], Ib_inv[3];
 };
 
+// knot-local input v of knot k -> column of x = [X(:) (12 N); jpos(:) (12 (N-1)); U(:) (24 (N-1))]
+KHD long long knot_col(int N, int k, int v) {
+  if (v < 12) return 12LL * k + v;
+  if (v < 24) return 12LL * N + 12LL * k + (v - 12);
+  if (v < 48) return 12LL * N + 12LL * (N - 1) + 24LL * k + (v - 24);
+  if (v < 60) return 12LL * (k + 1) + (v - 48);
+  return 12LL * N + 12LL * (N - 1) + 24LL * (k + 1) + (v - 60);
+}
+
 KHD double hip_x(int l) { return l < 2 ? 0.19 : -0.19; }      // hipSrbmLocation, get_robot_params.m:90-91
 KHD double hip_y(int l) { return (l & 1) ? 0.1 : -0.1; }
 KHD double side_y(int l) { return (l & 1) ? 1.0 : -1.0; }     // side_sign(2, leg) = sideSign of get_foot_jacobians_mc.m:3

@@ -1,7 +1,9 @@
-"""Times the kino-dynamic evaluation kernels (g, CCS Jacobian, upper-triangle Lagrangian Hessian; SURVEY 8 f-2) on
-device-resident SoA buffers: algorithmic bytes = 8 * (inputs read + outputs written) per scenario -- n_x + m for g,
-n_x + nnzJ for the Jacobian, n_x + m + nnzH (+ lam_f) for the Hessian -- against the HBM copy bandwidth measured in the
-same run.  At N = 21 and 16384 scenarios every input exceeds the 126 MB L2.
+"""Times the kino-dynamic evaluation kernels (g, CCS Jacobian, upper-triangle Lagrangian Hessian, Lagrangian gradient and
+KKT residuals; SURVEY 8 f-2) on device-resident SoA buffers: algorithmic bytes = 8 * (inputs read + outputs written) per
+scenario -- n_x + m for g, n_x + nnzJ for the Jacobian, n_x + m + nnzH (+ lam_f) for the Hessian, n_x + m + 1 + n_x for
+grad_x alone, and for all four KKT outputs that plus the bounds (2 m), the g the call computes (m) and the three scalars
+-- against the HBM copy bandwidth measured in the same run.  At N = 21 and 16384 scenarios every input exceeds the
+126 MB L2.
    usage: python tools/bench_kino.py [N] [B]        (prints one JSON line per function, with the card's name and power limit)"""
 import json
 import os
@@ -45,12 +47,16 @@ def measure_kino(N=21, B=16384, reps=10, solver=None, device=0, hess=False):
     x = torch.rand(d["nx"], B, dtype=torch.float64, device=dev) - 0.5
     g = torch.zeros(d["m"], B, dtype=torch.float64, device=dev)
     jac = torch.zeros(d["nnzJ"], B, dtype=torch.float64, device=dev)
-    nnzH = H = lam_f = lam_g = 0
+    nnzH = H = lam_f = lam_g = lbg = ubg = gx = sc = 0
     if hess:
         nnzH = len(s.kino_hess_sparsity()[1])
         lam_f = torch.ones(B, dtype=torch.float64, device=dev)
         lam_g = torch.randn(d["m"], B, dtype=torch.float64, device=dev)
         H = torch.zeros(nnzH, B, dtype=torch.float64, device=dev)
+        lbg = -torch.rand(d["m"], B, dtype=torch.float64, device=dev)
+        ubg = torch.rand(d["m"], B, dtype=torch.float64, device=dev)
+        gx = torch.zeros(d["nx"], B, dtype=torch.float64, device=dev)
+        sc = torch.zeros(3, B, dtype=torch.float64, device=dev)
     st = torch.cuda.ExternalStream(s.stream_ptr, device=dev)
     torch.cuda.synchronize()
     if hess:
@@ -61,8 +67,13 @@ def measure_kino(N=21, B=16384, reps=10, solver=None, device=0, hess=False):
     out = []
     calls = (("kino_g", lambda: s.kino_eval_device(x, pb, g=g), d["nx"] + d["m"]),
              ("kino_jac_g", lambda: s.kino_eval_device(x, pb, jac=jac), d["nx"] + d["nnzJ"]),
-             ("kino_hess_l", lambda: s.kino_hess_device(x, pb, H, lam_f=lam_f, lam_g=lam_g), d["nx"] + d["m"] + nnzH + 1))
-    for name, call, words in calls[:3 if hess else 2]:
+             ("kino_hess_l", lambda: s.kino_hess_device(x, pb, H, lam_f=lam_f, lam_g=lam_g), d["nx"] + d["m"] + nnzH + 1),
+             ("kino_grad_x", lambda: s.kino_kkt_device(x, pb, lam_f=lam_f, lam_g=lam_g, grad_x=gx),
+              2 * d["nx"] + d["m"] + 1),
+             ("kino_kkt", lambda: s.kino_kkt_device(x, pb, lam_f=lam_f, lam_g=lam_g, lbg=lbg, ubg=ubg, grad_x=gx,
+                                                    viol=sc[0], dual_inf=sc[1], compl_inf=sc[2]),
+              2 * d["nx"] + d["m"] + 1 + 3 * d["m"] + 3))
+    for name, call, words in calls[:5 if hess else 2]:
         for _ in range(3):
             call()
         s.synchronize()
