@@ -19,8 +19,9 @@ struct HostLam {
   double operator()(int row) const { return l ? l[row] : 0.0; }
 };
 
-extern "C" int hostcheck_eval(int N, const double* x, const double* p, double lam_f, const double* lam_g,
-                              double* g, double* jac, double* hes) {
+// cs == nullptr: formulation 0; else the SCHED instantiation (formulation 1) with cs[4 k + leg] of knot k
+static int eval_all(int N, const double* x, const double* p, double lam_f, const double* lam_g, const int* cs,
+                    double* g, double* jac, double* hes) {
   auto pl = get_plan(N);
   const ParamOff& o = pl->off;
   if (g) {
@@ -44,12 +45,27 @@ extern "C" int hostcheck_eval(int N, const double* x, const double* p, double la
     }
     kn.h = p[o.dt + k]; kn.mu = p[o.mu]; kn.mass = p[o.mass];
     for (int i = 0; i < 3; i++) { kn.Ib[i] = p[o.Ib + i]; kn.Ibinv[i] = p[o.Ibinv + i]; }
+    for (int l = 0; l < 4; l++) kn.csv[l] = cs ? (double)cs[4 * k + l] : 0.0;
     HostSink s{g ? g + 36 + 104 * k : nullptr, jac, hes, pl->jmap.data() + k * NJ_INT, pl->hmap.data() + k * NH_INT};
     HostLam lam{lam_g ? lam_g + 36 + 104 * k : nullptr};
-    if (last) knot_eval<true, true, true, true>(kn, s, lam);
-    else knot_eval<false, true, true, true>(kn, s, lam);
+    if (cs) {
+      if (last) knot_eval<true, true, true, true, HostSink, HostLam, true>(kn, s, lam);
+      else knot_eval<false, true, true, true, HostSink, HostLam, true>(kn, s, lam);
+    } else {
+      if (last) knot_eval<true, true, true, true>(kn, s, lam);
+      else knot_eval<false, true, true, true>(kn, s, lam);
+    }
   }
   return 0;
+}
+extern "C" int hostcheck_eval(int N, const double* x, const double* p, double lam_f, const double* lam_g,
+                              double* g, double* jac, double* hes) {
+  return eval_all(N, x, p, lam_f, lam_g, nullptr, g, jac, hes);
+}
+// the fixed-contact-schedule instantiation; the boundary rows 0..35 are filled as in hostcheck_eval
+extern "C" int hostcheck_eval_sched(int N, const double* x, const double* p, double lam_f, const double* lam_g,
+                                    const int* cs, double* g, double* jac, double* hes) {
+  return eval_all(N, x, p, lam_f, lam_g, cs, g, jac, hes);
 }
 extern "C" const long long* hostcheck_sparsity(int N, int which) {
   auto pl = get_plan(N);

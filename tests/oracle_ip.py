@@ -73,8 +73,10 @@ def default_problem(**kw):
     return pb
 
 
-def solve_cpu(N, drops, opt=None, pb=None, threads=0, fast=False):
-    """drops [B,12] -> dict(x [B,nx], status, iters, f, viol, n_factor).  fast: the -O3 -march=native build (timing only)."""
+def solve_cpu(N, drops, opt=None, pb=None, threads=0, fast=False, want_lam=False):
+    """drops [B,12] -> dict(x [B,nx], status, iters, f, viol, n_factor).  fast: the -O3 -march=native build (timing only).
+    want_lam: also lam_g [B,m]; the scenarios then go one at a time through ip_solve (which returns the multipliers) on
+    a pool of host threads, from the same initial guess as ip_solve_batch."""
     lib = _lib(fast)
     drops = np.ascontiguousarray(drops, dtype=np.float64)
     B = drops.shape[0]
@@ -84,14 +86,29 @@ def solve_cpu(N, drops, opt=None, pb=None, threads=0, fast=False):
     x = np.zeros((B, nx))
     res = (IpResult * B)()
     threads = min(threads or (os.cpu_count() or 1), max(B, 1))
-    rc = lib.ip_solve_batch(N, B, _dp(drops), ctypes.byref(pb), ctypes.byref(opt), _dp(x), res,
-                            threads or (os.cpu_count() or 1))
-    assert rc == 0
-    return dict(x=x, status=np.array([r.status for r in res]), iters=np.array([r.iters for r in res]),
-                f=np.array([r.f for r in res]), viol=np.array([r.viol for r in res]),
-                n_factor=np.array([r.n_factor for r in res]), mu=np.array([r.mu for r in res]),
-                dual_inf=np.array([r.dual_inf for r in res]), compl_inf=np.array([r.compl_inf for r in res]),
-                restarts=np.array([r.restarts for r in res]))
+    out = {}
+    if want_lam:
+        from concurrent.futures import ThreadPoolExecutor
+        from oracle_lib import Oracle
+        o = Oracle(N)
+        lam = np.zeros((B, o.m))
+
+        def one(b):  # (ctypes releases the GIL during the call)
+            p, x0 = o.build_p_x0(pb, drops[b, :6], drops[b, 6:])
+            lib.ip_solve(o.plan, _dp(p), _dp(x0), ctypes.byref(opt), _dp(x[b]), _dp(lam[b]), ctypes.byref(res[b]))
+
+        with ThreadPoolExecutor(threads) as ex:
+            list(ex.map(one, range(B)))
+        out["lam_g"] = lam
+    else:
+        rc = lib.ip_solve_batch(N, B, _dp(drops), ctypes.byref(pb), ctypes.byref(opt), _dp(x), res, threads)
+        assert rc == 0
+    out.update(x=x, status=np.array([r.status for r in res]), iters=np.array([r.iters for r in res]),
+               f=np.array([r.f for r in res]), viol=np.array([r.viol for r in res]),
+               n_factor=np.array([r.n_factor for r in res]), mu=np.array([r.mu for r in res]),
+               dual_inf=np.array([r.dual_inf for r in res]), compl_inf=np.array([r.compl_inf for r in res]),
+               restarts=np.array([r.restarts for r in res]))
+    return out
 
 
 def solve_cpu_x0(N, drops, x0, opt=None, pb=None):
