@@ -37,6 +37,7 @@ enum {
   LANDING_ST_LINESEARCH_FAIL = 2,
   LANDING_ST_NAN = 3,
   LANDING_ST_FACTOR_FAIL = 4,
+  LANDING_ST_NOT_INTERIOR = 5, /* landing_kino_step_batch: a slack or bound multiplier not strictly interior */
   LANDING_ST_RUNNING = 9
 };
 
@@ -217,7 +218,8 @@ int landing_tvlqr_batch(landing_ctx *ctx, long long B, int memspace, const landi
  * kinematics of the legs (get_forward_kin_foot.m:4-25), joint-torque limits tau = J_f' (-R' f) (get_foot_jacobians_mc.m:12-24),
  * joint limits, XYZ rotation convention (rpyToRotMat_xyz.m:2).  Batched constraint values and sparse Jacobian (CCS value
  * array, pattern from landing_kino_sparsity) and, below, the Lagrangian Hessian (landing_kino_hess_batch), gradient and
- * KKT residuals (landing_kino_kkt_batch) -- the functions an NLP solver iterates on; the interior-point kernel itself solves the SRB formulations only.  x[B x n_x] = [X(:); jpos(:); U(:)] per scenario (Opti variable order :45-51),
+ * KKT residuals (landing_kino_kkt_batch) -- the functions an NLP solver iterates on -- and the primal-dual Newton step of
+ * one interior-point iteration (landing_kino_step_batch); the interior-point loop over them is not part of the library.  x[B x n_x] = [X(:); jpos(:); U(:)] per scenario (Opti variable order :45-51),
  * g[B x m], jac[B x nnz]; dims = {N, n_x = 12N + 36(N-1), m = 48 + 141(N-2) + 117, nnz}.  The row map and the bounds
  * lbg / ubg are restated in oracle/kino_ref.py (pinned to the stored solution generate_solver/prevSoln.mat). */
 typedef struct landing_kino_problem {
@@ -292,6 +294,45 @@ typedef struct landing_kino_kkt_io {
  * the bounds. */
 int landing_kino_kkt_batch(landing_ctx *ctx, long long B, int memspace, int layout, const landing_kino_problem *pb,
                            const landing_kino_setup *ks, const landing_kino_kkt_io *io);
+
+/* Primal-dual Newton step of one interior-point iteration of the kino-dynamic NLP, with IPOPT's inertia correction, per
+ * scenario.  IPOPT's form (oracle/ip_ref.c): every inequality row i has a slack s_i and bound multipliers zL_i (finite
+ * lbg_i) and zU_i (finite ubg_i); y has CasADi's sign, L = f + y'(g - s); W = the hess of landing_kino_hess_batch with
+ * lam_f = 1, lam_g = y.  The step solves
+ *   (W + delta_w I) dx + J' dy       = -(grad_f + J' y)
+ *   -dy_i - dzL_i + dzU_i            = y_i + zL_i - zU_i         inequality rows
+ *   J_E dx                           = -(g_E - lbg_E)            equality rows
+ *   J_I dx - ds                      = -(g_I - s)
+ *   zL ds + (s - lbg) dzL            = mu - zL (s - lbg)         finite lbg
+ *   -zU ds + (ubg - s) dzU           = mu - zU (ubg - s)         finite ubg
+ * The row kinds are structural: the equality rows are rows 0..23 (X_0, c_0) and the 12 dynamics rows of each knot, every
+ * other row is an inequality row (one with both bounds infinite has y + dy = 0).  delta_w follows IPOPT's schedule from
+ * dw_last: the first trial is dw_last / 3 (0 if that is below 1e-7, or if dw_last = 0); after a failed factorisation
+ * 1e-4 (dw_last = 0) or max(1e-20, dw_last / 3), then x100 (at most 8 times while dw_last = 0) or x8; above 1e40 the
+ * scenario fails.  A factorisation fails when a Cholesky pivot of a stage's control block is <= 1e-14, which is exactly
+ * "the reduced Hessian on the null space of J_E is not positive definite".  Per scenario: status 0 (step found),
+ * LANDING_ST_FACTOR_FAIL or LANDING_ST_NOT_INTERIOR (a slack not strictly inside a finite bound of its row, or a
+ * multiplier of a finite bound <= 0): then every output vector of that scenario is NaN, and no other scenario is touched.
+ * delta_w: the value used (NaN for a non-interior iterate); n_factor: factorisations tried.  With tau in (0, 1) and the
+ * alpha outputs: the fraction-to-boundary step lengths alpha_pr = max a <= 1 with (s - lbg) + a ds >= (1 - tau)(s - lbg)
+ * and (ubg - s) - a ds >= (1 - tau)(ubg - s), alpha_du the same for zL + a dzL and zU + a dzU.  ds, dzL, dzU are 0 on
+ * equality rows and dzL / dzU on infinite bounds; s, zL, zU are not read there.  Results are the same bits in both
+ * layouts, both memory spaces and from run to run; every output entry is written on every call; B = 0 launches nothing. */
+typedef struct landing_kino_step_io {
+  const double *g, *jac, *hess, *grad_f; /* [B x m], [B x nnzJ], [B x nnzH], [B x n_x] at the iterate */
+  const double *s, *y, *zL, *zU;         /* [B x m] */
+  const double *lbg, *ubg;               /* [B x m] */
+  const double *mu, *dw_last;            /* [B] in both layouts */
+  double *dx;                            /* [B x n_x] */
+  double *ds, *dy, *dzL, *dzU;           /* [B x m] */
+  double *delta_w;                       /* [B] */
+  int *n_factor, *status;                /* [B] */
+  double tau;                            /* fraction-to-boundary parameter, needed with alpha_pr / alpha_du */
+  double *alpha_pr, *alpha_du;           /* [B], both or neither (optional) */
+} landing_kino_step_io;
+/* LANDING_ERR_ARG, with the context left usable: a NULL ctx / io / required pointer, B < 0, only one alpha output, or
+ * tau outside (0, 1) with the alpha outputs. */
+int landing_kino_step_batch(landing_ctx *ctx, long long B, int memspace, int layout, const landing_kino_step_io *io);
 
 /* Measured FP64 FMA throughput of the context's device in TFLOP/s (a DFMA micro-kernel timed with CUDA
  * events): the roofline denominator of the interior-point kernel, which is FP64-pipe bound by design. */

@@ -83,6 +83,13 @@ class KinoKktIO(ctypes.Structure):
     _fields_ = [(n, _dp) for n in ("x", "lam_f", "lam_g", "lbg", "ubg", "grad_x", "viol", "dual_inf", "compl_inf")]
 
 
+class KinoStepIO(ctypes.Structure):
+    """landing_kino_step_io: an interior-point iterate of the kino-dynamic NLP and its primal-dual Newton step."""
+    _fields_ = [(n, _dp) for n in ("g", "jac", "hess", "grad_f", "s", "y", "zL", "zU", "lbg", "ubg", "mu", "dw_last", "dx",
+                                   "ds", "dy", "dzL", "dzU", "delta_w")] + \
+        [("n_factor", _ip), ("status", _ip), ("tau", ctypes.c_double), ("alpha_pr", _dp), ("alpha_du", _dp)]
+
+
 class SolveIO(ctypes.Structure):
     _fields_ = [("drops", _dp), ("x0", _dp), ("x_star", _dp), ("f_star", _dp), ("lam_g", _dp),
                 ("viol", _dp), ("status", _ip), ("iters", _ip)]
@@ -131,6 +138,9 @@ def load_library(path=LIB_PATH):
         lib.landing_kino_kkt_batch.argtypes = [ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int, ctypes.c_int,
                                                ctypes.POINTER(KinoProblem), ctypes.POINTER(KinoSetup),
                                                ctypes.POINTER(KinoKktIO)]
+    if hasattr(lib, "landing_kino_step_batch"):
+        lib.landing_kino_step_batch.argtypes = [ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int, ctypes.c_int,
+                                                ctypes.POINTER(KinoStepIO)]
     lib.landing_launch_count.restype = ctypes.c_longlong
     lib.landing_launch_count.argtypes = [ctypes.c_void_p]
     if hasattr(lib, "landing_fp64_peak"):
@@ -527,6 +537,46 @@ class LandingSolver:
         self._check(self.lib.landing_kino_kkt_batch(self.ctx, B, DEVICE, layout, ctypes.byref(pb),
                                                     None if ks is None else ctypes.byref(ks), ctypes.byref(io)),
                     "landing_kino_kkt_batch")
+
+    STEP_IN = ("g", "jac", "hess", "grad_f", "s", "y", "zL", "zU", "lbg", "ubg")
+    STEP_OUT = ("dx", "ds", "dy", "dzL", "dzU")
+
+    def kino_step_host(self, g, jac, hess, grad_f, s, y, zL, zU, lbg, ubg, mu, dw_last, tau=None, layout=AOS):
+        """Primal-dual Newton step of one interior-point iteration of the kino-dynamic NLP (include/landing_b200.h:
+        landing_kino_step_batch).  Host arrays; layout SOA: [n, B] (mu, dw_last and the [B] outputs are [B] in both
+        layouts).  g, s, y, zL, zU, lbg, ubg [B, m]; jac [B, nnzJ] (landing_kino_eval_batch), hess [B, nnzH]
+        (landing_kino_hess_batch with lam_f = 1, lam_g = y), grad_f [B, n_x] (landing_kino_cost_batch).  tau in (0, 1):
+        also the fraction-to-boundary step lengths.  Returns a dict: dx, ds, dy, dzL, dzU, delta_w, n_factor, status
+        (and alpha_pr, alpha_du)."""
+        c = (lambda a: np.ascontiguousarray(a, dtype=np.float64))
+        ins = [c(a) for a in (g, jac, hess, grad_f, s, y, zL, zU, lbg, ubg)]
+        mu, dw_last = c(mu), c(dw_last)
+        B = mu.shape[0]
+        d = self.kino_dims()
+        shp = lambda n: (B, n) if layout == AOS else (n, B)  # noqa: E731
+        out = {"dx": np.zeros(shp(d["nx"]))}
+        for k in self.STEP_OUT[1:]:
+            out[k] = np.zeros(shp(d["m"]))
+        out.update(delta_w=np.zeros(B), n_factor=np.zeros(B, np.int32), status=np.zeros(B, np.int32))
+        if tau is not None:
+            out.update(alpha_pr=np.zeros(B), alpha_du=np.zeros(B))
+        io = KinoStepIO(*[_ptr(a) for a in ins], _ptr(mu), _ptr(dw_last), *[_ptr(out[k]) for k in self.STEP_OUT],
+                        _ptr(out["delta_w"]), _ptr(out["n_factor"], _ip), _ptr(out["status"], _ip),
+                        0.0 if tau is None else float(tau), _ptr(out.get("alpha_pr")), _ptr(out.get("alpha_du")))
+        self._check(self.lib.landing_kino_step_batch(self.ctx, B, HOST, layout, ctypes.byref(io)), "landing_kino_step_batch")
+        return out
+
+    def kino_step_device(self, inputs, outputs, tau=None, layout=SOA):
+        """Same with CUDA torch tensors already in HBM (enqueued on the library stream).  inputs: dict of g, jac, hess,
+        grad_f, s, y, zL, zU, lbg, ubg, mu, dw_last; outputs: dict of dx, ds, dy, dzL, dzU, delta_w, n_factor (int32),
+        status (int32) and, with tau, alpha_pr, alpha_du."""
+        B = inputs["mu"].shape[0]
+        io = KinoStepIO(*[_ptr(inputs[k]) for k in self.STEP_IN], _ptr(inputs["mu"]), _ptr(inputs["dw_last"]),
+                        *[_ptr(outputs[k]) for k in self.STEP_OUT], _ptr(outputs["delta_w"]),
+                        _ptr(outputs["n_factor"], _ip), _ptr(outputs["status"], _ip), 0.0 if tau is None else float(tau),
+                        _ptr(outputs.get("alpha_pr")), _ptr(outputs.get("alpha_du")))
+        self._check(self.lib.landing_kino_step_batch(self.ctx, B, DEVICE, layout, ctypes.byref(io)),
+                    "landing_kino_step_batch")
 
     def synchronize(self):
         self._check(self.lib.landing_synchronize(self.ctx), "landing_synchronize")

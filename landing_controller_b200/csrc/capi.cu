@@ -3,6 +3,7 @@
 // every entry point that produces numbers needs a CUDA device and fails loudly without one.
 #include <cstdio>
 #include <cstdlib>
+#include <algorithm>
 #include <cstring>
 #include <map>
 #include <memory>
@@ -64,6 +65,12 @@ struct landing_ctx {
   int* d_khess = nullptr;
   // scratch of its KKT residuals (landing_kino_kkt_batch): g, and grad_x when the caller does not ask for it
   DeviceBuf kkt;
+  // its interior-point Newton step (landing_kino_step_batch): plan tables + scenario counter, made on first use, and the
+  // factor scratch of the resident CTAs
+  std::shared_ptr<const KinoStepHost> kstep;
+  int* d_kstep = nullptr;
+  int kstep_grid = 0;
+  DeviceBuf kstep_scr;
 };
 
 // dt[0..N-2] of this call on the device (stream-ordered): the caller's vector or the uniform T/(N-1)
@@ -259,6 +266,7 @@ void landing_destroy(landing_ctx* c) {
   if (c->d_maps) cudaFree(c->d_maps);
   if (c->d_kino) cudaFree(c->d_kino);
   if (c->d_khess) cudaFree(c->d_khess);
+  if (c->d_kstep) cudaFree(c->d_kstep);
   delete c;  // (the grow-only buffers)
   if (st) cudaStreamDestroy(st);
 }
@@ -554,6 +562,75 @@ int landing_kino_kkt_batch(landing_ctx* c, long long B, int memspace, int layout
   soa_to_aos(c, B, pc, 5);
   CU(cudaGetLastError());
   return stage_out(c, memspace, pc, 9);
+}
+
+// Launches of one call (B > 0): 1 step kernel (k_kino_step), + for AoS batches of B >= 64 the transposes of the ten
+// [B x n] inputs and of the five [B x n] outputs: 1 (SoA, or AoS with B < 64) or 16 (AoS, B >= 64).
+int landing_kino_step_batch(landing_ctx* c, long long B, int memspace, int layout, const landing_kino_step_io* io) {
+  if (!c || !io || B < 0) return fail(LANDING_ERR_ARG, "landing_kino_step_batch: bad arguments");
+  const void* req[] = {io->g, io->jac, io->hess, io->grad_f, io->s, io->y, io->zL, io->zU, io->lbg, io->ubg, io->mu,
+                       io->dw_last, io->dx, io->ds, io->dy, io->dzL, io->dzU, io->delta_w, io->n_factor, io->status};
+  for (const void* p : req)
+    if (!p) return fail(LANDING_ERR_ARG, "landing_kino_step_batch: a required pointer is NULL");
+  if (!io->alpha_pr != !io->alpha_du)
+    return fail(LANDING_ERR_ARG, "landing_kino_step_batch: give both alpha_pr and alpha_du, or neither");
+  if (io->alpha_pr && !(io->tau > 0.0 && io->tau < 1.0))
+    return fail(LANDING_ERR_ARG, "landing_kino_step_batch: tau must be in (0, 1) with the alpha outputs");
+  if (B == 0) return LANDING_OK;
+  DeviceGuard guard_(c->device);
+  if (!c->kstep) {
+    auto hp = get_kino_hess_plan(c->N);
+    if (!hp->err.empty()) return fail(LANDING_ERR_ARG, hp->err);
+    auto pl = std::make_shared<KinoStepHost>();
+    const std::string err = make_kino_step_tables(c->N, get_kino_plan(c->N)->sparsity.data(), hp->sparsity.data(), pl.get());
+    if (!err.empty()) return fail(LANDING_ERR_ARG, err);
+    CU(cudaMalloc(&c->d_kstep, sizeof(int) * (pl->flat.size() + 1)));
+    CU(cudaMemcpy(c->d_kstep, pl->flat.data(), sizeof(int) * pl->flat.size(), cudaMemcpyHostToDevice));
+    cudaError_t e = cudaSuccess;
+    c->kstep_grid = kino_step_resident(&e);
+    CU(e);
+    c->kstep = pl;
+  }
+  const KinoStepHost& pl = *c->kstep;
+  const long long nx = pl.nx, m = pl.m, nnzJ = get_kino_plan(c->N)->nnz, nnzH = get_kino_hess_plan(c->N)->nnz;
+  // the [B x n] arrays of AoS batches on transposed copies (landing_kino_eval_batch); the others are [B]
+  Piece pc[22] = {input(io->g, m * B),    input(io->jac, nnzJ * B), input(io->hess, nnzH * B), input(io->grad_f, nx * B),
+                  input(io->s, m * B),    input(io->y, m * B),      input(io->zL, m * B),      input(io->zU, m * B),
+                  input(io->lbg, m * B),  input(io->ubg, m * B),    output(io->dx, nx * B),    output(io->ds, m * B),
+                  output(io->dy, m * B),  output(io->dzL, m * B),   output(io->dzU, m * B),    input(io->mu, B),
+                  input(io->dw_last, B),  output(io->delta_w, B),   output(io->n_factor, B),   output(io->status, B),
+                  output(io->alpha_pr, B), output(io->alpha_du, B)};
+  int rc = stage_in(c, memspace, pc, 22);
+  if (!rc) rc = aos_to_soa(c, B, &layout, pc, 15);
+  if (rc) return rc;
+  const int grid = (int)std::min<long long>(B, c->kstep_grid);
+  const long long slot = kino_step_slot(c->N);
+  CU(c->kstep_scr.reserve(sizeof(double) * slot * grid));
+  KinoStepArgs a{};
+  a.B = B;
+  a.tb = kino_step_view(pl, c->d_kstep);
+  const long long n[15] = {m, nnzJ, nnzH, nx, m, m, m, m, m, m, nx, m, m, m, m};
+  CView* in[10] = {&a.g, &a.jac, &a.hess, &a.grad_f, &a.s, &a.y, &a.zL, &a.zU, &a.lbg, &a.ubg};
+  View* out[5] = {&a.dx, &a.ds, &a.dy, &a.dzL, &a.dzU};
+  for (int i = 0; i < 10; i++) *in[i] = make_cview(pc[i].at<const double>(), n[i], B, layout);
+  for (int i = 0; i < 5; i++) *out[i] = make_view(pc[10 + i].at<double>(), n[10 + i], B, layout);
+  a.mu = make_cview(pc[15].at<const double>(), 1, B, layout);
+  a.dw_last = make_cview(pc[16].at<const double>(), 1, B, layout);
+  a.delta_w = make_view(pc[17].at<double>(), 1, B, layout);
+  a.n_factor = pc[18].at<int>();
+  a.status = pc[19].at<int>();
+  a.alpha_pr = make_view(pc[20].at<double>(), 1, B, layout);
+  a.alpha_du = make_view(pc[21].at<double>(), 1, B, layout);
+  a.tau = io->tau;
+  a.scratch = c->kstep_scr.as<double>();
+  a.slot = slot;
+  a.counter = c->d_kstep + pl.flat.size();
+  CU(cudaMemsetAsync(a.counter, 0, sizeof(int), c->stream));
+  c->launches += launch_kino_step(a, grid, c->stream);
+  CU(cudaGetLastError());
+  soa_to_aos(c, B, pc, 15);
+  CU(cudaGetLastError());
+  return stage_out(c, memspace, pc, 22);
 }
 
 int landing_fp64_peak(landing_ctx* c, double* tflops) {

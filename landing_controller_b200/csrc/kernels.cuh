@@ -7,6 +7,7 @@
 
 #include "../../include/landing_b200.h"
 #include "kino_knot.cuh"
+#include "kino_step.cuh"
 #include "plan.cuh"
 
 namespace srb {
@@ -131,6 +132,30 @@ struct KinoKktArgs {
   View viol, dual_inf, compl_inf;   // [1 x B], any may be NULL
 };
 int launch_kino_kkt(const KinoKktArgs& a, cudaStream_t st);
+// interior-point Newton step of the kino-dynamic NLP (kino_step.cu): the plan's tables (one flat int array, offsets of
+// the twelve StepTables arrays) and the launch
+struct KinoStepHost {
+  int N = 0;
+  long long nx = 0, m = 0, off[12] = {};
+  std::vector<int> flat;
+};
+std::string make_kino_step_tables(int N, const long long* jac_sparsity, const long long* hess_sparsity, KinoStepHost* out);
+kino::StepTables kino_step_view(const KinoStepHost& h, const int* dev);
+struct KinoStepArgs {
+  long long B;
+  kino::StepTables tb;
+  CView g, jac, hess, grad_f, s, y, zL, zU, lbg, ubg, mu, dw_last;
+  View dx, ds, dy, dzL, dzU, delta_w, alpha_pr, alpha_du;  // alpha_*: p NULL when not wanted
+  int *n_factor, *status;  // [B]
+  double tau;
+  double* scratch;  // [grid][slot]
+  long long slot;
+  int* counter;     // scenario counter (zeroed before the launch)
+};
+int kino_step_smem_bytes();
+long long kino_step_slot(int N);
+int kino_step_resident(cudaError_t* err);
+int launch_kino_step(const KinoStepArgs& a, int grid, cudaStream_t st);
 
 // returns number of kernel launches issued
 int launch_eval(const EvalArgs& a, cudaStream_t st);
