@@ -17,7 +17,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import kino_ref as kr  # noqa: E402
 from test_kino_exact import random_problem, random_x, kino_problem  # noqa: E402
 from test_kino_step_host import (harness, patterns, interior_point, full_system, fraction_to_boundary,  # noqa: E402,F401
-                                 run_host, ccs, eq_rows)
+                                 run_host, ccs, eq_rows, dw_trials)
 
 pytestmark = pytest.mark.gpu
 IN = ("g", "jac", "hess", "grad_f", "s", "y", "zL", "zU", "lbg", "ubg")
@@ -180,8 +180,10 @@ def test_gpu_step_first_iteration_from_the_srb_initial_guess():
 
 
 def test_gpu_step_failures_stay_in_their_scenario():
-    """A NaN in one scenario's Jacobian and a slack on its bound in another change nothing elsewhere (bit for bit); the
-    second reports LANDING_ST_NOT_INTERIOR with NaN outputs."""
+    """A NaN in one scenario's Jacobian and a slack on its bound in another change nothing elsewhere (bit for bit).  The
+    NaN is on an inequality row's entry in a control column of stage 1, so it reaches that stage's control block: the
+    first reports LANDING_ST_FACTOR_FAIL after the whole inertia schedule, the second LANDING_ST_NOT_INTERIOR; both
+    with NaN outputs."""
     import landing_controller_b200 as lc
     N, B = 4, 6
     s = lc.LandingSolver(N=N, device=0)
@@ -189,7 +191,10 @@ def test_gpu_step_failures_stay_in_their_scenario():
     inp = make_inputs(s, rng, N, B)
     clean = step(s, lc, inp, "SOA", "DEVICE")
     bad = {k: v.copy() for k, v in inp.items()}
-    bad["jac"][1, 17] = np.nan
+    colind, row = ccs(patterns(N)[0])
+    c = 12 * N + 12  # jpos_1[0], a control of stage 1
+    e = next(e for e in range(colind[c], colind[c + 1]) if not eq_rows(N)[row[e]])
+    bad["jac"][1, e] = np.nan
     i = np.flatnonzero(~eq_rows(N) & np.isfinite(inp["lbg"][4]))[5]
     bad["s"][4, i] = bad["lbg"][4, i]
     out = step(s, lc, bad, "SOA", "DEVICE")
@@ -200,7 +205,12 @@ def test_gpu_step_failures_stay_in_their_scenario():
     assert out["n_factor"][4] == 0 and np.isnan(out["delta_w"][4])
     for k in OUT:
         assert np.all(np.isnan(out[k][4])), k
-    assert out["status"][1] != 0 or not np.all(np.isfinite(out["dx"][1]))
+    trials = dw_trials(0.0, 100)
+    nf = next(i for i, d in enumerate(trials) if d > 1e40)
+    assert out["status"][1] == 4  # LANDING_ST_FACTOR_FAIL
+    assert out["n_factor"][1] == nf and out["delta_w"][1] == trials[nf]
+    for k in OUT + ("alpha_pr", "alpha_du"):
+        assert np.all(np.isnan(out[k][1])), k
 
 
 def test_gpu_step_refused_arguments_and_empty_batch():
