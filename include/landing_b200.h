@@ -218,8 +218,8 @@ int landing_tvlqr_batch(landing_ctx *ctx, long long B, int memspace, const landi
  * kinematics of the legs (get_forward_kin_foot.m:4-25), joint-torque limits tau = J_f' (-R' f) (get_foot_jacobians_mc.m:12-24),
  * joint limits, XYZ rotation convention (rpyToRotMat_xyz.m:2).  Batched constraint values and sparse Jacobian (CCS value
  * array, pattern from landing_kino_sparsity) and, below, the Lagrangian Hessian (landing_kino_hess_batch), gradient and
- * KKT residuals (landing_kino_kkt_batch) -- the functions an NLP solver iterates on -- and the primal-dual Newton step of
- * one interior-point iteration (landing_kino_step_batch); the interior-point loop over them is not part of the library.  x[B x n_x] = [X(:); jpos(:); U(:)] per scenario (Opti variable order :45-51),
+ * KKT residuals (landing_kino_kkt_batch) -- the functions an NLP solver iterates on --, the primal-dual Newton step of
+ * one interior-point iteration (landing_kino_step_batch) and the interior-point solve over them (landing_kino_solve_batch).  x[B x n_x] = [X(:); jpos(:); U(:)] per scenario (Opti variable order :45-51),
  * g[B x m], jac[B x nnz]; dims = {N, n_x = 12N + 36(N-1), m = 48 + 141(N-2) + 117, nnz}.  The row map and the bounds
  * lbg / ubg are restated in oracle/kino_ref.py (pinned to the stored solution generate_solver/prevSoln.mat). */
 typedef struct landing_kino_problem {
@@ -333,6 +333,46 @@ typedef struct landing_kino_step_io {
 /* LANDING_ERR_ARG, with the context left usable: a NULL ctx / io / required pointer, B < 0, only one alpha output, or
  * tau outside (0, 1) with the alpha outputs. */
 int landing_kino_step_batch(landing_ctx *ctx, long long B, int memspace, int layout, const landing_kino_step_io *io);
+
+/* Interior-point solve of the kino-dynamic NLP, one per drop condition: the second half of the reference's pipeline
+ * (main_scripts/landing_optimization.m:300-377: SRB solve, then the KNITRO kino-dynamic solve from its solution).  The
+ * method is IPOPT's primal-dual filter line search as oracle/ip_ref.c restates it for the SRB solver (DESIGN.md 3, 3.2):
+ * relaxed bounds, slacks on the inequality rows (the structural row kinds of landing_kino_step_batch), the monotone
+ * barrier update, the filter with switching condition and Armijo test, IPOPT's inertia correction, and the jamming
+ * watchdog with re-centring instead of a restoration phase.  The landing_options fields used keep their meanings
+ * (max_iter, tol, constr_viol_tol, dual_inf_tol, compl_inf_tol, mu_init, bound_push, bound_frac, bound_relax_factor,
+ * jam_iters, jam_alpha, max_restarts, restart_mu).  The bounds and, without x0, the initial guess are those of
+ * landing_kino_setup_batch for the drop (from x_srb, or from the reference trajectories when x_srb is NULL); the cost is
+ * the terminal cost of landing_kino_cost_batch.  Buffers are AoS, host or device per memspace.  Per scenario: status
+ * (CONVERGED, MAX_ITER, LINESEARCH_FAIL, NAN -- a NaN in the drop, the guess or any measured quantity --, FACTOR_FAIL),
+ * iters, x_star, f_star = f(x_star), and optionally lam_g (y, CasADi's sign), restarts and the final viol / dual_inf /
+ * compl_inf with the definitions of landing_kino_kkt_batch at (x_star, lam_f = 1, lam_g) and the bounds of the drop.
+ * A scenario's result is the same bits whether it is solved alone or in any batch, in any order, from host or device
+ * buffers.  The host synchronises the context's stream once per outer round and once per line-search round to read
+ * back a count; otherwise, with device buffers, the call only enqueues.  stats (HOST pointer, optional): outer rounds,
+ * line-search rounds and compactions of the call; the launch count is documented beside the call in capi.cu.
+ * MEMORY: the call keeps the state of all B scenarios on the device at once (two copies of the persistent state, the
+ * round's Jacobian, Hessian and direction, the trial point): about 0.73 MB per scenario at N = 21 and 1.41 MB at N = 40,
+ * in one allocation that grows with B.  There is no chunking: a batch whose scratch does not fit the device fails with
+ * LANDING_ERR_CUDA (the context stays usable); split such a batch into several calls. */
+typedef struct landing_kino_solve_io {
+  const double *drops; /* [B x 12] (q_init, qd_init), required */
+  const double *x_srb; /* [B x (36N-24)] SRB solutions (landing_solve_batch's x_star) or NULL */
+  const double *x0;    /* [B x n_x] initial guess or NULL: then the guess of landing_kino_setup_batch from x_srb */
+  double *x_star;      /* [B x n_x] */
+  double *f_star;      /* [B]      terminal cost at x_star */
+  double *lam_g;       /* [B x m]  y with CasADi's sign (L = f + lam_g' g), optional */
+  double *viol, *dual_inf, *compl_inf; /* [B] final measures (the definitions of landing_kino_kkt_batch), optional */
+  int *status, *iters; /* [B] */
+  int *restarts;       /* [B] re-centrings used, optional */
+  long long *stats;    /* [3] HOST: outer rounds, line-search rounds, compactions; optional */
+} landing_kino_solve_io;
+/* LANDING_ERR_ARG, with the context left usable: a NULL ctx / pb / pb->dt / ks / opt / io / drops / x_star / f_star /
+ * status / iters, B < 0, or options out of range (max_iter < 0, a tolerance, mu_init or bound_push <= 0, bound_frac
+ * outside (0, 0.5], bound_relax_factor < 0, jam_iters < 0, jam_alpha < 0, max_restarts < 0, restart_mu NaN).  B = 0
+ * launches nothing. */
+int landing_kino_solve_batch(landing_ctx *ctx, long long B, int memspace, const landing_kino_problem *pb,
+                             const landing_kino_setup *ks, const landing_options *opt, const landing_kino_solve_io *io);
 
 /* Measured FP64 FMA throughput of the context's device in TFLOP/s (a DFMA micro-kernel timed with CUDA
  * events): the roofline denominator of the interior-point kernel, which is FP64-pipe bound by design. */

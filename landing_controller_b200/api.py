@@ -90,6 +90,12 @@ class KinoStepIO(ctypes.Structure):
         [("n_factor", _ip), ("status", _ip), ("tau", ctypes.c_double), ("alpha_pr", _dp), ("alpha_du", _dp)]
 
 
+class KinoSolveIO(ctypes.Structure):
+    """landing_kino_solve_io: drop conditions (and SRB solutions or an initial guess) in, the kino-dynamic solutions out."""
+    _fields_ = [(n, _dp) for n in ("drops", "x_srb", "x0", "x_star", "f_star", "lam_g", "viol", "dual_inf", "compl_inf")] + \
+        [("status", _ip), ("iters", _ip), ("restarts", _ip), ("stats", ctypes.POINTER(ctypes.c_longlong))]
+
+
 class SolveIO(ctypes.Structure):
     _fields_ = [("drops", _dp), ("x0", _dp), ("x_star", _dp), ("f_star", _dp), ("lam_g", _dp),
                 ("viol", _dp), ("status", _ip), ("iters", _ip)]
@@ -141,6 +147,10 @@ def load_library(path=LIB_PATH):
     if hasattr(lib, "landing_kino_step_batch"):
         lib.landing_kino_step_batch.argtypes = [ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int, ctypes.c_int,
                                                 ctypes.POINTER(KinoStepIO)]
+    if hasattr(lib, "landing_kino_solve_batch"):
+        lib.landing_kino_solve_batch.argtypes = [ctypes.c_void_p, ctypes.c_longlong, ctypes.c_int,
+                                                 ctypes.POINTER(KinoProblem), ctypes.POINTER(KinoSetup),
+                                                 ctypes.POINTER(Options), ctypes.POINTER(KinoSolveIO)]
     lib.landing_launch_count.restype = ctypes.c_longlong
     lib.landing_launch_count.argtypes = [ctypes.c_void_p]
     if hasattr(lib, "landing_fp64_peak"):
@@ -577,6 +587,60 @@ class LandingSolver:
                         _ptr(outputs.get("alpha_pr")), _ptr(outputs.get("alpha_du")))
         self._check(self.lib.landing_kino_step_batch(self.ctx, B, DEVICE, layout, ctypes.byref(io)),
                     "landing_kino_step_batch")
+
+    KINO_SOLVE_OUT = ("lam_g", "viol", "dual_inf", "compl_inf", "restarts")
+
+    def kino_solve_host(self, drops, x_srb=None, x0=None, pb=None, ks=None, options=None, want=KINO_SOLVE_OUT):
+        """Interior-point solve of the kino-dynamic NLP for a batch of drop conditions [B, 12] (include/landing_b200.h:
+        landing_kino_solve_batch), from the SRB solutions x_srb [B, 36N-24] (landing_solve_batch's x) or an initial guess
+        x0 [B, n_x] (None: landing_kino_setup_batch's guess).  pb: kino_problem (default: the reference's dt for N = 21,
+        else uniform over 0.6 s); ks: kino_setup_data(); options: self.options.  Host arrays; returns a dict with x, f,
+        status, iters, stats (outer rounds, line-search rounds, compactions) and the optional outputs named in want."""
+        d = self.kino_dims()
+        drops = np.ascontiguousarray(drops, dtype=np.float64)
+        B = drops.shape[0]
+        c = (lambda a: None if a is None else np.ascontiguousarray(a, dtype=np.float64))
+        x_srb, x0 = c(x_srb), c(x0)
+        pb = pb or self._kino_default_problem()
+        ks = ks or self.kino_setup_data()
+        opt = options or self.options
+        out = dict(x=np.zeros((B, d["nx"])), f=np.zeros(B), status=np.full(B, 9, np.int32), iters=np.zeros(B, np.int32),
+                   stats=np.zeros(3, np.int64))
+        if "lam_g" in want:
+            out["lam_g"] = np.zeros((B, d["m"]))
+        for k in ("viol", "dual_inf", "compl_inf"):
+            if k in want:
+                out[k] = np.zeros(B)
+        if "restarts" in want:
+            out["restarts"] = np.zeros(B, np.int32)
+        io = KinoSolveIO(_ptr(drops), _ptr(x_srb), _ptr(x0), _ptr(out["x"]), _ptr(out["f"]), _ptr(out.get("lam_g")),
+                         _ptr(out.get("viol")), _ptr(out.get("dual_inf")), _ptr(out.get("compl_inf")),
+                         _ptr(out["status"], _ip), _ptr(out["iters"], _ip), _ptr(out.get("restarts"), _ip),
+                         _ptr(out["stats"], ctypes.POINTER(ctypes.c_longlong)))
+        self._check(self.lib.landing_kino_solve_batch(self.ctx, B, HOST, ctypes.byref(pb), ctypes.byref(ks),
+                                                      ctypes.byref(opt), ctypes.byref(io)), "landing_kino_solve_batch")
+        return out
+
+    def kino_solve_device(self, drops, x_star, f_star, status, iters, x_srb=None, x0=None, lam_g=None, viol=None,
+                          dual_inf=None, compl_inf=None, restarts=None, pb=None, ks=None, options=None):
+        """Same with CUDA torch tensors already in HBM (AoS, enqueued on the library stream; the call reads back one count
+        per outer round and per line-search round).  Returns stats (outer rounds, line-search rounds, compactions)."""
+        B = drops.shape[0]
+        pb = pb or self._kino_default_problem()
+        ks = ks or self.kino_setup_data()
+        opt = options or self.options
+        stats = np.zeros(3, np.int64)
+        io = KinoSolveIO(_ptr(drops), _ptr(x_srb), _ptr(x0), _ptr(x_star), _ptr(f_star), _ptr(lam_g), _ptr(viol),
+                         _ptr(dual_inf), _ptr(compl_inf), _ptr(status, _ip), _ptr(iters, _ip), _ptr(restarts, _ip),
+                         _ptr(stats, ctypes.POINTER(ctypes.c_longlong)))
+        self._check(self.lib.landing_kino_solve_batch(self.ctx, B, DEVICE, ctypes.byref(pb), ctypes.byref(ks),
+                                                      ctypes.byref(opt), ctypes.byref(io)), "landing_kino_solve_batch")
+        return stats
+
+    def _kino_default_problem(self):
+        """The reference's knot spacings for N = 21 (generate_landingCtrller_KNITRO.m:30), else uniform over 0.6 s."""
+        dt = [0.05] + [0.02] * 15 + [0.05, 0.05, 0.1, 0.2] if self.N == 21 else [0.6 / (self.N - 1)] * (self.N - 1)
+        return self.kino_problem(np.array(dt))
 
     def synchronize(self):
         self._check(self.lib.landing_synchronize(self.ctx), "landing_synchronize")

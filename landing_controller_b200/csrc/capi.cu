@@ -71,6 +71,10 @@ struct landing_ctx {
   int* d_kstep = nullptr;
   int kstep_grid = 0;
   DeviceBuf kstep_scr;
+  // its interior-point solve (landing_kino_solve_batch): state scratch (grows with B), counters + a device 1.0, and
+  // the pinned word of the per-round read-backs
+  DeviceBuf ksol, ksol_misc;
+  PinnedBuf ksol_count;
 };
 
 // dt[0..N-2] of this call on the device (stream-ordered): the caller's vector or the uniform T/(N-1)
@@ -375,21 +379,27 @@ int landing_kino_cost_batch(landing_ctx* c, long long B, int memspace, int layou
   return stage_out(c, memspace, pc, 3);
 }
 
+// the device tables of landing_kino_eval_batch's Jacobian scatter, made on first use
+static int ensure_kino_tables(landing_ctx* c) {
+  if (c->kino) return LANDING_OK;
+  auto pl = get_kino_plan(c->N);
+  const size_t n = pl->gpos.size() + pl->bpos.size();
+  CU(cudaMalloc(&c->d_kino, sizeof(int) * n));
+  CU(cudaMemcpy(c->d_kino, pl->gpos.data(), sizeof(int) * pl->gpos.size(), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(c->d_kino + pl->gpos.size(), pl->bpos.data(), sizeof(int) * pl->bpos.size(), cudaMemcpyHostToDevice));
+  c->kino = pl;
+  return LANDING_OK;
+}
+
 int landing_kino_eval_batch(landing_ctx* c, long long B, int memspace, int layout, const landing_kino_problem* pb,
                             const double* x, double* g, double* jac) {
   if (!c || !pb || !pb->dt || !x || B < 0) return fail(LANDING_ERR_ARG, "landing_kino_eval_batch: bad arguments");
   if (B == 0 || (!g && !jac)) return LANDING_OK;
   DeviceGuard guard_(c->device);
-  if (!c->kino) {
-    auto pl = get_kino_plan(c->N);
-    const size_t n = pl->gpos.size() + pl->bpos.size();
-    CU(cudaMalloc(&c->d_kino, sizeof(int) * n));
-    CU(cudaMemcpy(c->d_kino, pl->gpos.data(), sizeof(int) * pl->gpos.size(), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(c->d_kino + pl->gpos.size(), pl->bpos.data(), sizeof(int) * pl->bpos.size(), cudaMemcpyHostToDevice));
-    c->kino = pl;
-  }
+  int rc = ensure_kino_tables(c);
+  if (rc) return rc;
   const KinoPlan& pl = *c->kino;
-  int rc = stage_dt(c, pb->dt, 0.0);
+  rc = stage_dt(c, pb->dt, 0.0);
   if (rc) return rc;
   // AoS batches (one vector per scenario, what landing_solve_batch / landing_kino_setup_batch hand over) are evaluated
   // on transposed copies like the SRB functions (landing_eval_batch)
@@ -434,6 +444,21 @@ const long long* landing_kino_hess_sparsity(int N) {
   return pl->sparsity.data();
 }
 
+// the device tables of landing_kino_hess_batch (entry writers, terminal diagonal, row masks), made on first use
+static int ensure_kino_hess_tables(landing_ctx* c) {
+  if (c->khess) return LANDING_OK;
+  auto pl = get_kino_hess_plan(c->N);
+  if (!pl->err.empty()) return fail(LANDING_ERR_ARG, pl->err);
+  const size_t n = pl->hpos.size() + pl->cpos.size() + pl->rows.size();
+  CU(cudaMalloc(&c->d_khess, sizeof(int) * n));
+  CU(cudaMemcpy(c->d_khess, pl->hpos.data(), sizeof(int) * pl->hpos.size(), cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(c->d_khess + pl->hpos.size(), pl->cpos.data(), sizeof(int) * 12, cudaMemcpyHostToDevice));
+  CU(cudaMemcpy(c->d_khess + pl->hpos.size() + 12, pl->rows.data(), sizeof(unsigned) * pl->rows.size(),
+                cudaMemcpyHostToDevice));
+  c->khess = pl;
+  return LANDING_OK;
+}
+
 int landing_kino_hess_batch(landing_ctx* c, long long B, int memspace, int layout, const landing_kino_problem* pb,
                             const landing_kino_setup* ks, const double* x, const double* lam_f, const double* lam_g,
                             double* hess) {
@@ -441,20 +466,11 @@ int landing_kino_hess_batch(landing_ctx* c, long long B, int memspace, int layou
     return fail(LANDING_ERR_ARG, "landing_kino_hess_batch: bad arguments (lam_f needs ks)");
   if (B == 0) return LANDING_OK;
   DeviceGuard guard_(c->device);
-  if (!c->khess) {
-    auto pl = get_kino_hess_plan(c->N);
-    if (!pl->err.empty()) return fail(LANDING_ERR_ARG, pl->err);
-    const size_t n = pl->hpos.size() + pl->cpos.size() + pl->rows.size();
-    CU(cudaMalloc(&c->d_khess, sizeof(int) * n));
-    CU(cudaMemcpy(c->d_khess, pl->hpos.data(), sizeof(int) * pl->hpos.size(), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(c->d_khess + pl->hpos.size(), pl->cpos.data(), sizeof(int) * 12, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(c->d_khess + pl->hpos.size() + 12, pl->rows.data(), sizeof(unsigned) * pl->rows.size(),
-                  cudaMemcpyHostToDevice));
-    c->khess = pl;
-  }
+  int rc = ensure_kino_hess_tables(c);
+  if (rc) return rc;
   const KinoHessPlan& pl = *c->khess;
   const long long m = 48 + 141LL * (c->N - 2) + 117;
-  int rc = stage_dt(c, pb->dt, 0.0);
+  rc = stage_dt(c, pb->dt, 0.0);
   if (rc) return rc;
   // x, lam_g and hess of AoS batches on transposed copies (landing_kino_eval_batch); lam_f is [B] in both layouts
   Piece pc[4] = {input(x, pl.nx * B), input(lam_g, m * B), output(hess, pl.nnz * B), input(lam_f, B)};
@@ -564,6 +580,23 @@ int landing_kino_kkt_batch(landing_ctx* c, long long B, int memspace, int layout
   return stage_out(c, memspace, pc, 9);
 }
 
+// the device tables of landing_kino_step_batch (plan + scenario counter) and its resident CTAs, made on first use
+static int ensure_kino_step_tables(landing_ctx* c) {
+  if (c->kstep) return LANDING_OK;
+  auto hp = get_kino_hess_plan(c->N);
+  if (!hp->err.empty()) return fail(LANDING_ERR_ARG, hp->err);
+  auto pl = std::make_shared<KinoStepHost>();
+  const std::string err = make_kino_step_tables(c->N, get_kino_plan(c->N)->sparsity.data(), hp->sparsity.data(), pl.get());
+  if (!err.empty()) return fail(LANDING_ERR_ARG, err);
+  CU(cudaMalloc(&c->d_kstep, sizeof(int) * (pl->flat.size() + 1)));
+  CU(cudaMemcpy(c->d_kstep, pl->flat.data(), sizeof(int) * pl->flat.size(), cudaMemcpyHostToDevice));
+  cudaError_t e = cudaSuccess;
+  c->kstep_grid = kino_step_resident(&e);
+  CU(e);
+  c->kstep = pl;
+  return LANDING_OK;
+}
+
 // Launches of one call (B > 0): 1 step kernel (k_kino_step), + for AoS batches of B >= 64 the transposes of the ten
 // [B x n] inputs and of the five [B x n] outputs: 1 (SoA, or AoS with B < 64) or 16 (AoS, B >= 64).
 int landing_kino_step_batch(landing_ctx* c, long long B, int memspace, int layout, const landing_kino_step_io* io) {
@@ -578,19 +611,7 @@ int landing_kino_step_batch(landing_ctx* c, long long B, int memspace, int layou
     return fail(LANDING_ERR_ARG, "landing_kino_step_batch: tau must be in (0, 1) with the alpha outputs");
   if (B == 0) return LANDING_OK;
   DeviceGuard guard_(c->device);
-  if (!c->kstep) {
-    auto hp = get_kino_hess_plan(c->N);
-    if (!hp->err.empty()) return fail(LANDING_ERR_ARG, hp->err);
-    auto pl = std::make_shared<KinoStepHost>();
-    const std::string err = make_kino_step_tables(c->N, get_kino_plan(c->N)->sparsity.data(), hp->sparsity.data(), pl.get());
-    if (!err.empty()) return fail(LANDING_ERR_ARG, err);
-    CU(cudaMalloc(&c->d_kstep, sizeof(int) * (pl->flat.size() + 1)));
-    CU(cudaMemcpy(c->d_kstep, pl->flat.data(), sizeof(int) * pl->flat.size(), cudaMemcpyHostToDevice));
-    cudaError_t e = cudaSuccess;
-    c->kstep_grid = kino_step_resident(&e);
-    CU(e);
-    c->kstep = pl;
-  }
+  if (int rc = ensure_kino_step_tables(c)) return rc;
   const KinoStepHost& pl = *c->kstep;
   const long long nx = pl.nx, m = pl.m, nnzJ = get_kino_plan(c->N)->nnz, nnzH = get_kino_hess_plan(c->N)->nnz;
   // the [B x n] arrays of AoS batches on transposed copies (landing_kino_eval_batch); the others are [B]
@@ -631,6 +652,79 @@ int landing_kino_step_batch(landing_ctx* c, long long B, int memspace, int layou
   soa_to_aos(c, B, pc, 15);
   CU(cudaGetLastError());
   return stage_out(c, memspace, pc, 22);
+}
+
+// Launches of one call (B > 0), with R outer rounds, S line-search rounds and C compactions (io->stats):
+//   25 R + 5 S + 3 C - 14, + 1 when io->x0 is given.
+// (start: set-up, g, f, init = 4; per outer round: grad_x 6 + KKT measures 1 + measure 1 + scan 1 = 9; per round that
+// takes a step, i.e. all but the last: Jacobian 8 + cost gradient 1 + Hessian 3 + step 1 + fraction to the boundary 1 +
+// the scan that ends its line search 1 + accept 1 = 16; per line-search round: scan 1 + trial 1 + g 1 + f 1 + filter 1
+// = 5; per compaction: output 1 + 2 gathers, and the last compaction, which leaves nothing running, has no gathers.)
+int landing_kino_solve_batch(landing_ctx* c, long long B, int memspace, const landing_kino_problem* pb,
+                             const landing_kino_setup* ks, const landing_options* opt, const landing_kino_solve_io* io) {
+  if (!c || !pb || !pb->dt || !ks || !opt || !io || B < 0)
+    return fail(LANDING_ERR_ARG, "landing_kino_solve_batch: bad arguments");
+  if (!io->drops || !io->x_star || !io->f_star || !io->status || !io->iters)
+    return fail(LANDING_ERR_ARG, "landing_kino_solve_batch: a required pointer is NULL");
+  const landing_options& o = *opt;
+  if (o.max_iter < 0 || !(o.tol > 0) || !(o.constr_viol_tol > 0) || !(o.dual_inf_tol > 0) || !(o.compl_inf_tol > 0) ||
+      !(o.mu_init > 0) || !(o.bound_push > 0) || !(o.bound_frac > 0 && o.bound_frac <= 0.5) ||
+      !(o.bound_relax_factor >= 0) || o.jam_iters < 0 || !(o.jam_alpha >= 0) || o.max_restarts < 0 ||
+      o.restart_mu != o.restart_mu)
+    return fail(LANDING_ERR_ARG, "landing_kino_solve_batch: options out of range");
+  if (io->stats) io->stats[0] = io->stats[1] = io->stats[2] = 0;
+  if (B == 0) return LANDING_OK;
+  DeviceGuard guard_(c->device);
+  int rc = ensure_kino_tables(c);
+  if (!rc) rc = ensure_kino_hess_tables(c);
+  if (!rc) rc = ensure_kino_step_tables(c);
+  if (!rc) rc = stage_dt(c, pb->dt, 0.0);
+  if (rc) return rc;
+  const KinoPlan& kp = *c->kino;
+  const KinoHessPlan& hp = *c->khess;
+  const KinoStepHost& sp = *c->kstep;
+  const long long nx = kp.nx, m = kp.m, nsrb = 36LL * c->N - 24;
+  Piece pc[12] = {input(io->drops, 12 * B),     input(io->x_srb, nsrb * B),  input(io->x0, nx * B),
+                  output(io->x_star, nx * B),   output(io->f_star, B),       output(io->lam_g, m * B),
+                  output(io->viol, B),          output(io->dual_inf, B),     output(io->compl_inf, B),
+                  output(io->status, B),        output(io->iters, B),        output(io->restarts, B)};
+  rc = stage_in(c, memspace, pc, 12);
+  if (rc) return rc;
+  const int grid = (int)std::min<long long>(B, c->kstep_grid);
+  const long long slot = kino_step_slot(c->N);
+  CU(c->kstep_scr.reserve(sizeof(double) * slot * grid));
+  CU(c->ksol.reserve((size_t)kino_solve_bytes(c->N, kp.nnz, hp.nnz) * (size_t)B));
+  if (!c->ksol_count.as<int>()) {
+    CU(c->ksol_misc.reserve(2 * sizeof(int) + sizeof(double)));
+    CU(c->ksol_count.reserve(sizeof(int)));
+    const double one = 1.0;
+    CU(cudaMemcpy(c->ksol_misc.as<char>() + 2 * sizeof(int), &one, sizeof(double), cudaMemcpyHostToDevice));
+  }
+  KinoSolveArgs a{};
+  a.N = c->N; a.B = B; a.nx = nx; a.m = m; a.nnzJ = kp.nnz; a.nnzH = hp.nnz;
+  a.pr = kino::Params{pb->mu, pb->mass, {pb->Ib[0], pb->Ib[1], pb->Ib[2]}, {pb->Ib_inv[0], pb->Ib_inv[1], pb->Ib_inv[2]}};
+  a.ks = *ks;
+  a.opt = o;
+  a.dtv = c->d_dt.as<double>();
+  a.gpos = c->d_kino; a.bpos = c->d_kino + kp.gpos.size();
+  a.hpos = c->d_khess; a.cpos = c->d_khess + hp.hpos.size();
+  a.hrows = reinterpret_cast<const unsigned*>(c->d_khess + hp.hpos.size() + 12);
+  a.tb = kino_step_view(sp, c->d_kstep);
+  a.step_grid = c->kstep_grid; a.step_scr = c->kstep_scr.as<double>(); a.step_slot = slot;
+  a.counter = c->ksol_misc.as<int>();
+  a.ones = reinterpret_cast<const double*>(c->ksol_misc.as<char>() + 2 * sizeof(int));
+  a.scratch = c->ksol.as<double>();
+  a.host_count = c->ksol_count.as<int>();
+  a.drops = pc[0].at<const double>(); a.x_srb = pc[1].at<const double>(); a.x0 = pc[2].at<const double>();
+  a.x_star = pc[3].at<double>(); a.f_star = pc[4].at<double>(); a.lam_g = pc[5].at<double>();
+  a.viol = pc[6].at<double>(); a.dual_inf = pc[7].at<double>(); a.compl_inf = pc[8].at<double>();
+  a.status = pc[9].at<int>(); a.iters = pc[10].at<int>(); a.restarts = pc[11].at<int>();
+  long long stats[3] = {0, 0, 0};
+  std::string err;
+  rc = kino_solve_run(a, c->stream, &c->launches, stats, &err);
+  if (rc) return fail(rc, "landing_kino_solve_batch: " + err);
+  if (io->stats) for (int i = 0; i < 3; i++) io->stats[i] = stats[i];
+  return stage_out(c, memspace, pc, 12);
 }
 
 int landing_fp64_peak(landing_ctx* c, double* tflops) {

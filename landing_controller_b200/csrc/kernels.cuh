@@ -156,6 +156,31 @@ int kino_step_smem_bytes();
 long long kino_step_slot(int N);
 int kino_step_resident(cudaError_t* err);
 int launch_kino_step(const KinoStepArgs& a, int grid, cudaStream_t st);
+// interior-point solve of the kino-dynamic NLP (kino_solve.cu): the host loop over the launchers above
+struct KinoSolveArgs {
+  int N;
+  long long B, nx, m, nnzJ, nnzH;
+  kino::Params pr;
+  landing_kino_setup ks;
+  landing_options opt;
+  const double* dtv;                       // knot spacings (device)
+  const int *gpos, *bpos;                  // launch_kino tables
+  const int *hpos, *cpos;                  // launch_kino_hess tables
+  const unsigned* hrows;
+  kino::StepTables tb;                     // launch_kino_step tables, resident CTAs, factor scratch
+  int step_grid;
+  double* step_scr;
+  long long step_slot;
+  int* counter;                            // [2]: the step's scenario counter, the scan count
+  const double* ones;                      // a device 1.0 (lam_f)
+  double* scratch;                         // kino_solve_bytes(N, nnzJ, nnzH) x B
+  int* host_count;                         // pinned host int (read-backs)
+  const double *drops, *x_srb, *x0;        // caller's buffers (AoS, device)
+  double *x_star, *f_star, *lam_g, *viol, *dual_inf, *compl_inf;
+  int *status, *iters, *restarts;
+};
+long long kino_solve_bytes(int N, long long nnzJ, long long nnzH);  // scratch bytes per scenario
+int kino_solve_run(const KinoSolveArgs& a, cudaStream_t st, long long* launches, long long stats[3], std::string* err);
 
 // returns number of kernel launches issued
 int launch_eval(const EvalArgs& a, cudaStream_t st);
